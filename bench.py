@@ -21,6 +21,11 @@ Two metrics (BASELINE.json names both), selected with --metric:
   --impl reference  the reference arm: the reference graph restated on the CPU (oracle/, torch fp32, all host
       cores; Chainer 7 is not installable in this image -- probed at run time, kind "port") on a bounded sample per
       step, same metric / config as the B200 arm.
+
+  --dump-outputs DIR  after the timed steps, what the last one computed, as DIR/<name>.npy: inference writes
+      continent_sample (2^23 seeded pixels of the 18000 x 22000 DEM inside its NaN frame); train writes train_metrics
+      (d_loss, d_accuracy, g_loss, g_psnr, g_ssim) and 2^22 seeded parameters of each model after that step. The inputs
+      are seeded, so two builds run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -155,6 +160,28 @@ def max_over_ranks(ms, world):
 def rel_l2(a, b):
     a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
     return float(np.linalg.norm(a - b) / (np.linalg.norm(b) + 1e-300))
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def seeded_sample(t, n, seed=0):
+    """``t`` flattened to the host if it has at most ``n`` elements, else ``n`` of its elements at fixed, seeded
+    positions in ascending order: the same positions on every run, so two builds compare element for element."""
+    flat = t.reshape(-1)
+    if flat.numel() <= n:
+        return flat.cpu().numpy()
+    idx = np.sort(np.random.RandomState(seed).randint(0, flat.numel(), size=n))
+    return flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes each array as <out_dir>/<name>.npy."""
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -539,12 +566,20 @@ def run_inference(args, rank, world, local):
     with ClockSampler(local) as clocks:
         e0.record()
         for _ in range(args.steps):
-            step()
+            y_hat = step()
         e1.record()
         barrier(world)
     launches = _lib.kernel_launches() - l0   # counted inside the library, one per kernel launch
     ms = max_over_ranks(e0.elapsed_time(e1), world)
     value = mpx * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # the DEM is 1.58 GB: 2^23 seeded pixels of the part the tiles write (their abutting windows), not of the
+        # frame the reference leaves NaN, which nothing computes
+        plan = tiler.tile_plan(final_shape, kw["ary_shape"], kw["stride"], kw["xtrapad"])
+        ys, ye = min(t[4] for t in plan), max(t[5] for t in plan)
+        xs, xe = min(t[6] for t in plan), max(t[7] for t in plan)
+        dump_outputs(args.dump_outputs, {"continent_sample": seeded_sample(y_hat[0, ys:ye, xs:xe], 1 << 23)})
+    del y_hat
 
     # every rank runs the instrumented strip (predict_continent ends in a collective); rank 0's CUDA-event timings
     # are the ones reported
@@ -659,7 +694,7 @@ def train_kernel_strip(step_fn, n_steps=2):
     return agg, n_steps
 
 
-def train_bench(rank, world, local, steps=50, warmup=5, batch=128, cpu=False, peak_tf=None):
+def train_bench(rank, world, local, steps=50, warmup=5, batch=128, cpu=False, peak_tf=None, dump_dir=None):
     from deepbedmap_b200 import _lib
     from deepbedmap_b200 import train as T
     if peak_tf is None:
@@ -673,9 +708,9 @@ def train_bench(rank, world, local, steps=50, warmup=5, batch=128, cpu=False, pe
 
     # the per-minibatch body of trainer() (srgan_train.py:1286-1308): both steps on the same device batch,
     # the generator step reusing the graph-keeping forward the discriminator step ran (weights unchanged between)
-    def eager_step():
-        T.train_eval_discriminator(arrays, g, d, d_opt, share_generator_forward=True)
-        T.train_eval_generator(arrays, g, d, g_opt)
+    def eager_step():   # returns the five metrics as GraphedTrainStep.step does
+        return (T.train_eval_discriminator(arrays, g, d, d_opt, share_generator_forward=True),
+                T.train_eval_generator(arrays, g, d, g_opt))
 
     launch = "CUDA graph replay (deepbedmap_b200.train.GraphedTrainStep)"
     graphed = None
@@ -693,11 +728,15 @@ def train_bench(rank, world, local, steps=50, warmup=5, batch=128, cpu=False, pe
     with ClockSampler(local) as clocks:
         e0.record()
         for _ in range(steps):
-            step()
+            metrics = step()
         e1.record()
         barrier(world)
     ms = max_over_ranks(e0.elapsed_time(e1), world) / steps
     eager_launches = None
+    if dump_dir and rank == 0:   # before the end-to-end steps below train the models further
+        dump_outputs(dump_dir, {"train_metrics": np.array([*metrics[0], *metrics[1]], np.float64),
+                                "generator_params_sample": seeded_sample(g.flat, 1 << 22),
+                                "discriminator_params_sample": seeded_sample(d.flat, 1 << 22)})
 
     # ---- end to end: a fresh pinned HOST minibatch per step -> H2D -> step -> five metrics back on the host ----
     host_batches = [{k: torch.rand(*s).pin_memory() for k, s in shapes.items()} for _ in range(4)]
@@ -779,7 +818,8 @@ def train_bench(rank, world, local, steps=50, warmup=5, batch=128, cpu=False, pe
 def run_train(args, rank, world, local):
     peak_tf, _, peak_src = measured_peaks()
     do_cpu = (not args.no_cpu) and world == 1
-    line = train_bench(rank, world, local, steps=args.steps, warmup=max(args.warmup, 3), cpu=do_cpu, peak_tf=peak_tf)
+    line = train_bench(rank, world, local, steps=args.steps, warmup=max(args.warmup, 3), cpu=do_cpu, peak_tf=peak_tf,
+                       dump_dir=args.dump_outputs)
     line["roofline_peak_source"] = peak_src
     if rank == 0:
         print(json.dumps(line))
@@ -803,9 +843,16 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64, "
+                         "a fixed seeded sample of outputs too large to keep whole, at most 64 MB in all)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 2 if args.metric == "inference" else 50
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     if args.impl == "reference":
         return run_reference(args)
     if args.warmup < 3:

@@ -29,6 +29,43 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from oracle import deepbedmap_oracle as O  # noqa: E402
 
 OUT = os.path.join(HERE, "hotpath_golden.npz")
+# No stored file exceeds 1 MB: a golden set named <name>.npz is written as shards <name>.<i>.npz of whole arrays, at
+# most SHARD_BYTES of array data each (the float data hardly compresses), and read back merged.
+SHARD_BYTES = 900_000
+
+
+def shard_path(path: str, i: int) -> str:
+    return f"{path[:-len('.npz')]}.{i}.npz"
+
+
+def save_golden(path: str, arrays: dict) -> list:
+    shards, size = [{}], 0
+    for k, v in arrays.items():
+        if v.nbytes > SHARD_BYTES:
+            raise ValueError(f"{k}: {v.nbytes} bytes do not fit one shard")
+        if shards[-1] and size + v.nbytes > SHARD_BYTES:
+            shards.append({})
+            size = 0
+        shards[-1][k] = v
+        size += v.nbytes
+    for i, s in enumerate(shards):
+        np.savez_compressed(shard_path(path, i), **s)
+    i = len(shards)
+    while os.path.exists(shard_path(path, i)):   # left over from a larger set
+        os.remove(shard_path(path, i))
+        i += 1
+    return [shard_path(path, i) for i in range(len(shards))]
+
+
+def load_golden(path: str) -> dict:
+    out, i = {}, 0
+    while os.path.exists(shard_path(path, i)):
+        with np.load(shard_path(path, i)) as z:
+            out.update({k: z[k] for k in z.files})
+        i += 1
+    if not out:
+        raise FileNotFoundError(f"no shards of {path}")
+    return out
 
 # (name, num_residual_blocks, batch, h, w, regime, HeNormal scale, bias_std)
 GENERATOR_CASES = [
@@ -156,13 +193,13 @@ def compute() -> dict:
 def main():
     if "--tiles" in sys.argv or "--all" in sys.argv:
         tiles = compute_tiles()
-        np.savez_compressed(TILE_OUT, **tiles)
-        print(f"wrote {TILE_OUT}: {len(tiles)} arrays, {os.path.getsize(TILE_OUT)} bytes")
+        files = save_golden(TILE_OUT, tiles)
+        print(f"wrote {len(tiles)} arrays to {files}")
         if "--all" not in sys.argv:
             return
     out = compute()
-    np.savez_compressed(OUT, **out)
-    print(f"wrote {OUT}: {len(out)} arrays, {os.path.getsize(OUT)} bytes")
+    files = save_golden(OUT, out)
+    print(f"wrote {len(out)} arrays to {files}")
 
 
 if __name__ == "__main__":

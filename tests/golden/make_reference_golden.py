@@ -185,8 +185,8 @@ def compute() -> dict:
 
 def main():
     out = compute()
-    np.savez_compressed(OUT, **out)
-    print(f"wrote {OUT}: {len(out)} arrays, {os.path.getsize(OUT)} bytes")
+    files = MG.save_golden(OUT, out)
+    print(f"wrote {len(out)} arrays to {files}")
 
 
 if __name__ == "__main__":

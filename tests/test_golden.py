@@ -23,8 +23,7 @@ O = MG.O
 
 @pytest.fixture(scope="module")
 def golden():
-    with np.load(MG.OUT) as z:
-        return {k: z[k] for k in z.files}
+    return MG.load_golden(MG.OUT)
 
 
 def rel_l2(a, b):

@@ -13,6 +13,7 @@ spread (the synthetic weights are random, so the raw output unit is arbitrary: m
 800 m being the standard deviation of the synthetic bed-elevation input X; run with -s to see them, the GPU log of
 the round is committed under profiles/).
 """
+import importlib.util
 import os
 
 import numpy as np
@@ -24,7 +25,10 @@ pytestmark = pytest.mark.gpu
 from oracle import deepbedmap_oracle as O  # noqa: E402  (test infrastructure)
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-GOLD = os.path.join(HERE, "golden", "continent_tiles_golden.npz")
+_spec = importlib.util.spec_from_file_location("make_golden", os.path.join(HERE, "golden", "make_golden.py"))
+MG = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(MG)
+GOLD = MG.TILE_OUT
 GRID, FINAL, STRIDE = (752, 752), (3000, 3000), 3
 STEM_PHYSICAL_SCALE = {"X": 1e-3, "W1": 5e-4, "W2": 5e-3, "W3": 2e-3}
 CASES = {  # name -> (tile index, HeNormal scale, bias_std, stem filters scaled to metre-valued inputs)
@@ -48,7 +52,7 @@ def grids():
 
 @pytest.fixture(scope="module")
 def gold():
-    return np.load(GOLD)
+    return MG.load_golden(GOLD)
 
 
 def make_model(scale, bias_std, physical, precision, nb=12):

@@ -8,24 +8,26 @@ to the reference-executed ones value by value.
 
 CPU only; nothing here reads /root/reference (the vectors are committed).
 """
+import importlib.util
 import os
 
 import numpy as np
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+_spec = importlib.util.spec_from_file_location("make_golden", os.path.join(HERE, "golden", "make_golden.py"))
+MG = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(MG)
 
 
 @pytest.fixture(scope="module")
 def ref():
-    with np.load(os.path.join(HERE, "golden", "reference_graph_golden.npz")) as z:
-        return {k: z[k] for k in z.files}
+    return MG.load_golden(os.path.join(HERE, "golden", "reference_graph_golden.npz"))
 
 
 @pytest.fixture(scope="module")
 def ora():
-    with np.load(os.path.join(HERE, "golden", "hotpath_golden.npz")) as z:
-        return {k: z[k] for k in z.files}
+    return MG.load_golden(MG.OUT)
 
 
 def rel_l2(a, b):
