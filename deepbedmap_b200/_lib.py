@@ -99,6 +99,22 @@ SIGNATURES = {
     "dbm_gen_set_precision": [_P, _I],
     "dbm_gen_workspace_bytes": [_P, _I, _I, _I],
     "dbm_gen_forward": [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P, ctypes.c_size_t, _P],
+    "dbm_disc_create": [ctypes.POINTER(_P)],
+    "dbm_disc_destroy": [_P],
+    "dbm_disc_set_precision": [_P, _I],
+    "dbm_disc_count_params": [_P],
+    "dbm_disc_num_arrays": [_P],
+    "dbm_disc_array_info": [_P, _I, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(_I), ctypes.POINTER(_I),
+                            ctypes.POINTER(_L)],
+    "dbm_disc_set_param": [_P, ctypes.c_char_p, _P, _I, ctypes.POINTER(_I)],
+    "dbm_disc_get_param": [_P, ctypes.c_char_p, _P],
+    "dbm_disc_bind_params": [_P, _P],
+    "dbm_disc_bind_grads": [_P, _P],
+    "dbm_disc_mark_updated": [_P],
+    "dbm_disc_zero_grads": [_P, _P],
+    "dbm_disc_workspace_bytes": [_P, _I],
+    "dbm_disc_forward": [_P, _P, _I, _I, _I, _I, _P, _P, ctypes.c_size_t, _P],
+    "dbm_disc_backward": [_P, _P, _P, ctypes.c_size_t, _P],
 }
 # tuning / A-B switches (include/deepbedmap_b200_tuning.h): exported by the same library, not part of the boundary
 TUNING_SIGNATURES = {
@@ -108,7 +124,8 @@ TUNING_SIGNATURES = {
     "dbm_local_debug_set": [_I],
 }
 # entry points that return a value instead of a status
-RESTYPES = {"dbm_launch_count": _L, "dbm_gen_count_params": _L, "dbm_gen_num_arrays": _I, "dbm_gen_workspace_bytes": ctypes.c_size_t}
+RESTYPES = {"dbm_launch_count": _L, "dbm_gen_count_params": _L, "dbm_gen_num_arrays": _I, "dbm_gen_workspace_bytes": ctypes.c_size_t,
+            "dbm_disc_count_params": _L, "dbm_disc_num_arrays": _I, "dbm_disc_workspace_bytes": ctypes.c_size_t}
 
 _lib: Optional[ctypes.CDLL] = None
 launch_count = 0  # number of library calls that enqueue kernels (bench.py reports it)

@@ -15,7 +15,7 @@ LIB = os.path.join(HERE, "libdeepbedmap_b200.so")
 TUNING_LIB = os.path.join(HERE, "libdeepbedmap_b200_tuning.so")
 STAMP = os.path.join(HERE, "build", "stamp.txt")
 
-SOURCES = ["ops.cu", "gemm_f32.cu", "gemm_bf16.cu", "umma_conv3x3.cu", "umma_trunk.cu", "umma_flat.cu", "umma_local.cu", "umma_deform.cu", "stem.cu", "deform_f32.cu", "train_ops.cu", "gen_api.cu"]
+SOURCES = ["ops.cu", "gemm_f32.cu", "gemm_bf16.cu", "umma_conv3x3.cu", "umma_trunk.cu", "umma_flat.cu", "umma_local.cu", "umma_deform.cu", "stem.cu", "deform_f32.cu", "train_ops.cu", "gen_api.cu", "disc_api.cu"]
 TUNING_SOURCES = ["debug_bench.cu"]   # libdeepbedmap_b200_tuning.so: microbenchmarks, never loaded by the product
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-Xcompiler", "-fPIC"]

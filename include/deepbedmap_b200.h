@@ -352,7 +352,8 @@ int dbm_gather_rows_f32(const float* src, long src_rows, const long* index_dev, 
  *     dbm_gen_array_info lists them in file order) -> dbm_gen_workspace_bytes -> dbm_gen_forward.
  * The handle owns the fp32 master weights (device; or views a caller-owned flat device buffer of
  * dbm_gen_count_params floats in App. C order, dbm_gen_bind_params), their re-packed bf16 UMMA operand images and
- * the pass table of the persistent trunk kernel -- the only device memory this library ever allocates. Activations
+ * the pass table of the persistent trunk kernel -- with the discriminator handle's (below), the only device memory this
+ * library allocates besides the deterministic mode's scratch. Activations
  * live in the caller's `workspace` (device, 1024-byte aligned, dbm_gen_workspace_bytes(n, h, w) bytes); everything is
  * enqueued on `stream`. Arithmetic: the tensor-core inference path (bf16 operands, fp32 accumulation, fp32 residual
  * stream; conv_on_W1 as a split-bf16 GEMM) or, after dbm_gen_set_precision(gen, 1), the split-bf16 path;
@@ -377,6 +378,49 @@ int dbm_gen_set_precision(dbm_gen* gen, int precision);
 size_t dbm_gen_workspace_bytes(const dbm_gen* gen, int n, int h, int w);
 int dbm_gen_forward(dbm_gen* gen, const float* x, const float* w1, const float* w2, const float* w3, int n, int h,
                     int w, float* y_out, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
+/* ---- model-level entry points: DiscriminatorModel (srgan_train.py:591-699) without the Python shim ---------------
+ * A host in any language runs the discriminator's training forward, backward and BatchNormalization bookkeeping with
+ *     dbm_disc_create -> dbm_disc_set_param (every array of the Chainer .npz: dbm_disc_array_info lists the 33
+ *     parameters in flat-buffer order, then avg_mean / avg_var / N of batch_norm1..9) -> dbm_disc_workspace_bytes ->
+ *     per step: dbm_disc_zero_grads -> dbm_disc_forward(train = 1, save = 1) -> loss gradient -> dbm_disc_backward.
+ * The handle owns the fp32 master weights and gradients (device; or views caller-owned flat device buffers of
+ * dbm_disc_count_params floats in layout.discriminator_shapes() order, dbm_disc_bind_params / dbm_disc_bind_grads: how
+ * an optimizer such as dbm_adam_step_f32 reaches them), the running statistics (device) and the nine N counters (host,
+ * kept as loaded: Chainer counts only in finetune mode, which the reference never enters), the packed bf16 operand
+ * images of conv_layer1..9 and every device table. x (n,1,36,36), logits (n,1), dlogit (n,1), the workspace (device,
+ * 1024-byte aligned, dbm_disc_workspace_bytes(n) bytes) and the stream belong to the caller.
+ *   forward: `groups` independent BatchNormalization batches stacked along n (D(real) | D(fake), srgan_train.py:
+ *     1145-1146; n % groups == 0); train = 1: batch statistics, running statistics updated group after group
+ *     (eps 1e-5, decay 0.9); train = 0: running statistics. save = 1 (needs train = 1) keeps in the workspace what
+ *     backward needs; a later forward on the same workspace discards it.
+ *   backward: accumulates d(loss)/d(params) into the gradient buffer (Chainer semantics: zero it per step) for the saved
+ *     pass of that workspace, and consumes it. Two passes in flight = two workspaces.
+ * Arithmetic: precision 0 (default) = conv_layer1..9 on the tcgen05 tensor cores (bf16 operands, fp32 accumulation;
+ * DiscriminatorModel(precision="bf16")), 1 = fp32 CUDA-core convolutions ("fp32"); conv_layer0, BatchNormalization,
+ * LeakyReLU and the Linear layers are fp32 in both. Results equal the Python class's bit for bit (gradients: under
+ * dbm_set_deterministic(1)). The first forward on a new (workspace, n, precision) uploads its tables and synchronises
+ * the stream once; later calls only enqueue (CUDA-graph capturable). A handle is bound to the device current at
+ * creation and is not thread-safe. dbm_disc_get_param / _set_param copy synchronously (no stream). */
+typedef struct dbm_disc dbm_disc;
+int dbm_disc_create(dbm_disc** out);
+int dbm_disc_destroy(dbm_disc* disc);
+/* 0 = bf16 tensor-core convolutions (default), 1 = fp32; changes dbm_disc_workspace_bytes and drops saved passes */
+int dbm_disc_set_precision(dbm_disc* disc, int precision);
+long dbm_disc_count_params(const dbm_disc* disc);           /* 10 370 761 (srgan_train.py:607-608) */
+int dbm_disc_num_arrays(const dbm_disc* disc);              /* 60: 33 parameters + 27 BatchNormalization persistents */
+/* flat_offset: position in the parameter buffer, -1 for the persistents; N has ndim 0 */
+int dbm_disc_array_info(const dbm_disc* disc, int index, const char** key, int* ndim, int* dims4, long* flat_offset);
+int dbm_disc_set_param(dbm_disc* disc, const char* key, const float* host_values, int ndim, const int* dims);
+int dbm_disc_get_param(const dbm_disc* disc, const char* key, float* host_values);   /* parameters and persistents */
+int dbm_disc_bind_params(dbm_disc* disc, float* device_flat);
+int dbm_disc_bind_grads(dbm_disc* disc, float* device_flat);   /* drops saved passes */
+int dbm_disc_mark_updated(dbm_disc* disc);                  /* after writing into a bound parameter buffer */
+int dbm_disc_zero_grads(dbm_disc* disc, cudaStream_t stream);  /* Link.cleargrads(), srgan_train.py:1162 */
+size_t dbm_disc_workspace_bytes(const dbm_disc* disc, int n);
+int dbm_disc_forward(dbm_disc* disc, const float* x, int n, int groups, int train, int save, float* logits,
+                     void* workspace, size_t workspace_bytes, cudaStream_t stream);
+int dbm_disc_backward(dbm_disc* disc, const float* dlogit, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
 #ifdef __cplusplus
 }
