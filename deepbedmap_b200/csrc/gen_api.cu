@@ -7,6 +7,7 @@
 // activations live in the caller's workspace; all work is enqueued on the caller's stream. The forward is the
 // tensor-core inference path (bf16 operands, fp32 accumulation, fp32 residual stream): the same kernels, in the same
 // order, with the same tables as deepbedmap_b200/model.py builds for its tiled path -- which now calls this file.
+#include <algorithm>
 #include <cstring>
 #include <map>
 #include <string>
@@ -23,8 +24,16 @@ struct GenParam {
   long off, n;
 };
 
-struct ImageRef {   // a packed bf16 operand image inside the arena
-  size_t off = 0;   // bytes
+// The packed operand images of one precision in one device arena, and the table dbm_pack_conv3x3_table executes to
+// (re)build them from the master weights
+struct PackArena {
+  uint8_t* base = nullptr;
+  PackEntry* dev = nullptr;   // pack table
+  int n = 0;                  // its entries
+  long max = 0;               // elements of the largest image
+  bool stale = true;          // the master weights changed since the last pack
+  std::map<std::string, size_t> img;   // image offsets by name
+  const __nv_bfloat16* image(const std::string& name) const { return (const __nv_bfloat16*)(base + img.at(name)); }
 };
 
 struct Gen {
@@ -36,26 +45,13 @@ struct Gen {
   long total = 0;
   float* flat = nullptr;     // device fp32 master weights, App. C order
   bool owns_flat = false;
-  // re-packed operands
-  uint8_t* arena = nullptr;
-  size_t arena_bytes = 0;
-  PackEntry* pack_dev = nullptr;
-  int pack_n = 0;
-  long pack_max = 0;
-  bool stale = true;
-  // offsets into the arena
-  std::map<std::string, size_t> img;     // packed images by name
+  // re-packed bf16 operands, and offsets of the stem / head regions of that arena
+  PackArena pack;
   size_t off_wts = 0, off_bias128 = 0, off_w1tc = 0, off_bias_off1 = 0, off_bias_off2 = 0;
   // precision: 0 = bf16 tensor-core path, 1 = "bf16x3" (split-bf16 trunk + upsample convs, fp32 stem and deformable
   // layers; dbm_gen_set_precision). The split operand images live in their own arena, built on first use.
   int precision = 0;
-  uint8_t* arena_s = nullptr;
-  size_t arena_s_bytes = 0;
-  PackEntry* pack_s_dev = nullptr;
-  int pack_s_n = 0;
-  long pack_s_max = 0;
-  bool stale_s = true;
-  std::map<std::string, size_t> img_s;
+  PackArena pack_s;
   // pass-table cache: rebuilt when the workspace or the shape changes
   const void* tab_ws = nullptr;
   int tab_n = 0, tab_h = 0, tab_w = 0, tab_layers = 0, tab_precision = -1;
@@ -121,83 +117,122 @@ static std::string rdb_prefix(int i, int r) {
   return "residual_network/" + std::to_string(i) + "/residual_dense_block" + std::to_string(r);
 }
 
-// Lays the packed operand images out in one arena and writes the table dbm_pack_conv3x3_table executes.
-static int build_pack_plan(Gen* g) {
+// Lays packed operand images out in an arena and collects the entries of its pack table. elem: bf16 elements of an
+// image per filter element (1, or 3 for split-bf16's [w_hi | w_hi | w_lo]); mode: the pack mode of every entry.
+struct PackPlan {
+  const Gen* g;
+  PackArena& a;
+  int elem, mode;
   std::vector<PackEntry> ent;
   size_t off = 0;
-  auto image = [&](const std::string& name, int cin, int coutp) {
-    g->img[name] = off;
-    off += ((size_t)9 * cin * coutp * 2 + 255) & ~(size_t)255;
-    return g->img[name];
-  };
-  auto entry = [&](const std::string& wkey, size_t img_off, int O, int o0, int cin, int cin_total, int c0, int coutp,
-                   int ck) {
-    PackEntry e;
-    e.w = P(g, wkey);
-    e.out = (__nv_bfloat16*)img_off;   // arena-relative for now, rebased after the allocation
-    e.O = O; e.o0 = o0; e.Cin = cin; e.CinTotal = cin_total; e.c0 = c0; e.COUTP = coutp; e.CK = ck; e.mode = 0;
-    ent.push_back(e);
-  };
-  const int ic = g->inter;
-  entry("pre_residual_conv_layer/W", image("pre", 128, 64), 64, 0, 128, 128, 0, 64, 16);
-  for (int i = 0; i < g->nb; ++i)
-    for (int r = 1; r <= 3; ++r) {
-      const std::string pre = rdb_prefix(i, r);
-      for (int k = 1; k <= 4; ++k) {
-        const int cin = 64 + (k - 1) * ic;
-        entry(pre + "/conv_layer" + std::to_string(k) + "/W", image(pre + "/c" + std::to_string(k), cin, ic), ic, 0, cin,
-              cin, 0, ic, 16);
-      }
-      entry(pre + "/conv_layer5/W", image(pre + "/c5", 64 + 4 * ic, 64), 64, 0, 64 + 4 * ic, 64 + 4 * ic, 0, 64, 16);
-      if (ic == 32)
-        for (int k = 1; k <= 3; k += 2) {   // dense-block pairing: head = conv_k | conv_{k+1} over shared inputs, tail
-          const int cin = 64 + (k - 1) * 32;
-          const std::string wa = pre + "/conv_layer" + std::to_string(k) + "/W";
-          const std::string wb = pre + "/conv_layer" + std::to_string(k + 1) + "/W";
-          const size_t both = image(pre + "/pair" + std::to_string(k), cin, 64);
-          entry(wa, both, 32, 0, cin, cin, 0, 64, 16);
-          entry(wb, both, 32, 32, cin, cin + 32, 0, 64, 16);
-          entry(wb, image(pre + "/tail" + std::to_string(k + 1), 32, 32), 32, 0, 32, cin + 32, cin, 32, 16);
-        }
-    }
-  entry("post_residual_conv_layer/W", image("post", 64, 64), 64, 0, 64, 64, 0, 64, 16);
-  entry("post_upsample_conv_layer_1/W", image("up1", 64, 64), 64, 0, 64, 64, 0, 64, 32);
-  entry("post_upsample_conv_layer_2/W", image("up2", 64, 64), 64, 0, 64, 64, 0, 64, 32);
-  entry("final_conv_layer1/offset_conv/W", image("off1", 64, 32), 18, 0, 64, 64, 0, 32, 32);
-  entry("final_conv_layer2/offset_conv/W", image("off2", 64, 32), 18, 0, 64, 64, 0, 32, 32);
-  entry("final_conv_layer1/deform_conv/W", image("dc1", 64, 64), 64, 0, 64, 64, 0, 64, 64);
-  auto raw = [&](size_t bytes) {
+  size_t raw(size_t bytes) {
     const size_t o = off;
     off += (bytes + 255) & ~(size_t)255;
     return o;
-  };
-  g->off_wts = raw(90 * 32 * 4);
-  g->off_bias128 = raw(128 * 4);
-  g->off_w1tc = raw((size_t)9 * 320 * 32 * 2);
-  g->off_bias_off1 = raw(32 * 4);
-  g->off_bias_off2 = raw(32 * 4);
-  g->arena_bytes = off;
-  DBM_CUDA(cudaMalloc(&g->arena, g->arena_bytes));
-  DBM_CUDA(cudaMemset(g->arena, 0, g->arena_bytes));   // padded rows / biases stay zero
-  long mx = 0;
-  for (auto& e : ent) {
-    e.out = (__nv_bfloat16*)(g->arena + (size_t)e.out);
-    const long el = (long)9 * e.Cin * e.COUTP;
-    if (el > mx) mx = el;
   }
-  g->pack_n = (int)ent.size();
-  g->pack_max = mx;
-  DBM_CUDA(cudaMalloc(&g->pack_dev, ent.size() * sizeof(PackEntry)));
-  DBM_CUDA(cudaMemcpy(g->pack_dev, ent.data(), ent.size() * sizeof(PackEntry), cudaMemcpyHostToDevice));
+  size_t image(const std::string& name, int cin, int coutp) {
+    return a.img[name] = raw((size_t)elem * 9 * cin * coutp * 2);
+  }
+  void entry(const std::string& wkey, size_t img_off, int O, int o0, int cin, int cin_total, int c0, int coutp, int ck) {
+    PackEntry e;
+    e.w = P(g, wkey);
+    e.out = (__nv_bfloat16*)img_off;   // arena-relative until upload()
+    e.O = O; e.o0 = o0; e.Cin = cin; e.CinTotal = cin_total; e.c0 = c0; e.COUTP = coutp; e.CK = ck; e.mode = mode;
+    ent.push_back(e);
+  }
+};
+
+// The trunk's filters in 16-channel chunks: pre-residual conv; per dense block conv1..4 (plain_dense), conv5 and, for
+// inter_channels 32, the pair / tail images of dense-block pairing (layout.trunk_plan); post-residual conv
+static void trunk_pack_entries(PackPlan& p, bool plain_dense) {
+  const int ic = p.g->inter, cc = 64 + 4 * ic;
+  p.entry("pre_residual_conv_layer/W", p.image("pre", 128, 64), 64, 0, 128, 128, 0, 64, 16);
+  for (int i = 0; i < p.g->nb; ++i)
+    for (int r = 1; r <= 3; ++r) {
+      const std::string pre = rdb_prefix(i, r);
+      for (int k = 1; plain_dense && k <= 4; ++k) {
+        const int cin = 64 + (k - 1) * ic;
+        p.entry(pre + "/conv_layer" + std::to_string(k) + "/W", p.image(pre + "/c" + std::to_string(k), cin, ic), ic, 0,
+                cin, cin, 0, ic, 16);
+      }
+      p.entry(pre + "/conv_layer5/W", p.image(pre + "/c5", cc, 64), 64, 0, cc, cc, 0, 64, 16);
+      if (ic == 32)
+        for (int k = 1; k <= 3; k += 2) {   // head = conv_k | conv_{k+1} over their shared inputs, tail = conv_{k+1} over a_k
+          const int cin = 64 + (k - 1) * 32;
+          const std::string wa = pre + "/conv_layer" + std::to_string(k) + "/W";
+          const std::string wb = pre + "/conv_layer" + std::to_string(k + 1) + "/W";
+          const size_t both = p.image(pre + "/pair" + std::to_string(k), cin, 64);
+          p.entry(wa, both, 32, 0, cin, cin, 0, 64, 16);
+          p.entry(wb, both, 32, 32, cin, cin + 32, 0, 64, 16);
+          p.entry(wb, p.image(pre + "/tail" + std::to_string(k + 1), 32, 32), 32, 0, 32, cin + 32, cin, 32, 16);
+        }
+    }
+  p.entry("post_residual_conv_layer/W", p.image("post", 64, 64), 64, 0, 64, 64, 0, 64, 16);
+}
+
+// Allocates the arena (zeroed: padded rows and biases stay zero), rebases the entries onto it and uploads the table
+static int upload(PackPlan& p) {
+  PackArena& a = p.a;
+  DBM_CUDA(cudaMalloc(&a.base, p.off));
+  DBM_CUDA(cudaMemset(a.base, 0, p.off));
+  a.max = 0;
+  for (auto& e : p.ent) {
+    e.out = (__nv_bfloat16*)(a.base + (size_t)e.out);
+    a.max = std::max(a.max, (long)9 * e.Cin * e.COUTP);
+  }
+  a.n = (int)p.ent.size();
+  DBM_CUDA(cudaMalloc(&a.dev, p.ent.size() * sizeof(PackEntry)));
+  DBM_CUDA(cudaMemcpy(a.dev, p.ent.data(), p.ent.size() * sizeof(PackEntry), cudaMemcpyHostToDevice));
+  a.stale = true;
   return DBM_OK;
 }
 
-static int refresh_packed(Gen* g, cudaStream_t st) {
-  if (!g->stale) return DBM_OK;
-  int rc = dbm_pack_conv3x3_table(g->pack_dev, g->pack_n, g->pack_max, st);
+// Points the table's filter pointers at a new master-weight buffer
+static int rebase_weights(PackArena& a, const float* from, const float* to) {
+  if (!a.dev) return DBM_OK;
+  std::vector<PackEntry> ent(a.n);
+  DBM_CUDA(cudaMemcpy(ent.data(), a.dev, ent.size() * sizeof(PackEntry), cudaMemcpyDeviceToHost));
+  for (auto& e : ent) e.w = to + (e.w - from);
+  DBM_CUDA(cudaMemcpy(a.dev, ent.data(), ent.size() * sizeof(PackEntry), cudaMemcpyHostToDevice));
+  return DBM_OK;
+}
+
+static int refresh(PackArena& a, cudaStream_t st) {
+  if (!a.stale) return DBM_OK;
+  const int rc = dbm_pack_conv3x3_table(a.dev, a.n, a.max, st);
   if (rc) return rc;
-  float* wts = (float*)(g->arena + g->off_wts);
-  float* bias128 = (float*)(g->arena + g->off_bias128);
+  a.stale = false;
+  return DBM_OK;
+}
+
+static void free_arena(PackArena& a) {
+  if (a.base) cudaFree(a.base);
+  if (a.dev) cudaFree(a.dev);
+}
+
+// The bf16 arena: the trunk's images, the upsample / offset / first deformable convs, and the stem's and heads' operands
+static int build_pack_plan(Gen* g) {
+  PackPlan p{g, g->pack, 1, 0};
+  trunk_pack_entries(p, true);
+  p.entry("post_upsample_conv_layer_1/W", p.image("up1", 64, 64), 64, 0, 64, 64, 0, 64, 32);
+  p.entry("post_upsample_conv_layer_2/W", p.image("up2", 64, 64), 64, 0, 64, 64, 0, 64, 32);
+  p.entry("final_conv_layer1/offset_conv/W", p.image("off1", 64, 32), 18, 0, 64, 64, 0, 32, 32);
+  p.entry("final_conv_layer2/offset_conv/W", p.image("off2", 64, 32), 18, 0, 64, 64, 0, 32, 32);
+  p.entry("final_conv_layer1/deform_conv/W", p.image("dc1", 64, 64), 64, 0, 64, 64, 0, 64, 64);
+  g->off_wts = p.raw(90 * 32 * 4);
+  g->off_bias128 = p.raw(128 * 4);
+  g->off_w1tc = p.raw((size_t)9 * 320 * 32 * 2);
+  g->off_bias_off1 = p.raw(32 * 4);
+  g->off_bias_off2 = p.raw(32 * 4);
+  return upload(p);
+}
+
+static int refresh_packed(Gen* g, cudaStream_t st) {
+  if (!g->pack.stale) return DBM_OK;
+  uint8_t* arena = g->pack.base;
+  float* wts = (float*)(arena + g->off_wts);
+  float* bias128 = (float*)(arena + g->off_bias128);
+  int rc;
   // conv_on_X (9 taps) | conv_on_W2 (72) | conv_on_W3 (9), tap-major [taps][32]
   if ((rc = dbm_transpose_f32(P(g, "input_block/conv_on_X/W"), wts, 32, 9, st))) return rc;
   if ((rc = dbm_transpose_f32(P(g, "input_block/conv_on_W2/W"), wts + 9 * 32, 32, 72, st))) return rc;
@@ -206,13 +241,12 @@ static int refresh_packed(Gen* g, cudaStream_t st) {
   for (int i = 0; i < 4; ++i)
     DBM_CUDA(cudaMemcpyAsync(bias128 + 32 * i, P(g, std::string("input_block/conv_on_") + stem[i] + "/b"), 32 * 4,
                              cudaMemcpyDeviceToDevice, st));
-  DBM_CUDA(cudaMemcpyAsync(g->arena + g->off_bias_off1, P(g, "final_conv_layer1/offset_conv/b"), 18 * 4,
+  DBM_CUDA(cudaMemcpyAsync(arena + g->off_bias_off1, P(g, "final_conv_layer1/offset_conv/b"), 18 * 4,
                            cudaMemcpyDeviceToDevice, st));
-  DBM_CUDA(cudaMemcpyAsync(g->arena + g->off_bias_off2, P(g, "final_conv_layer2/offset_conv/b"), 18 * 4,
+  DBM_CUDA(cudaMemcpyAsync(arena + g->off_bias_off2, P(g, "final_conv_layer2/offset_conv/b"), 18 * 4,
                            cudaMemcpyDeviceToDevice, st));
-  if ((rc = dbm_pack_stem_w1(P(g, "input_block/conv_on_W1/W"), g->arena + g->off_w1tc, st))) return rc;
-  g->stale = false;
-  return DBM_OK;
+  if ((rc = dbm_pack_stem_w1(P(g, "input_block/conv_on_W1/W"), arena + g->off_w1tc, st))) return rc;
+  return refresh(g->pack, st);   // the filter images, last: it clears the stale mark
 }
 
 // ---- workspace layout ------------------------------------------------------------------------------------------
@@ -253,31 +287,33 @@ static WsLayout ws_layout(const Gen* g, int n, int h, int w) {
   return L;
 }
 
-// Pass table of the persistent trunk kernel (the C++ twin of model.py's _trunk_workspace)
-static void build_trunk_table(Gen* g, const WsLayout& L, uint8_t* ws) {
-  std::vector<TrunkLayer>& T = g->tab_host;
+static void add_pass(std::vector<TrunkLayer>& T, const __nv_bfloat16* wq, const float* bias, int cin, int cout, int in_map,
+                     int act, float beta, __nv_bfloat16* out, int out_cs_total, int out_cs0, float* out_f32,
+                     const float* res1, const float* res2, int up2, int in_cs0, int cout_main, int mode) {
+  TrunkLayer t;
+  memset(&t, 0, sizeof(t));
+  t.wpacked = wq; t.bias = bias; t.out_bf16 = out; t.out_f32 = out_f32; t.res1 = res1; t.res2 = res2;
+  t.stash_out = nullptr;
+  t.cin = cin; t.cout = cout; t.in_map = in_map; t.in_cs0 = in_cs0; t.act = act; t.up2 = up2;
+  t.out_cs_total = out_cs_total; t.out_cs0 = out_cs0; t.cout_main = cout_main; t.res1_cs_total = 16;
+  t.beta = beta; t.mode = mode;
+  T.push_back(t);
+}
+
+// Pass table of the trunk kernels with the filter images of arena a and the buffers of workspace layout L (WsLayout or
+// WsSplit; cs fields are logical, the same for both): the C++ twin of layout.trunk_plan as model.py's
+// _trunk_workspace / _split_workspace bind it
+template <class Layout>
+static void build_trunk_passes(const Gen* g, const PackArena& a, const Layout& L, uint8_t* ws, std::vector<TrunkLayer>& T) {
   T.clear();
   auto bf = [&](size_t o) { return (__nv_bfloat16*)(ws + o); };
   auto f32 = [&](size_t o) { return (float*)(ws + o); };
-  auto image = [&](const std::string& name) { return (const __nv_bfloat16*)(g->arena + g->img.at(name)); };
-  auto layer = [&](const __nv_bfloat16* wq, const float* bias, int cin, int cout, int in_map, int act, float beta,
-                   __nv_bfloat16* out, int out_cs_total, int out_cs0, float* out_f32, const float* res1,
-                   const float* res2, int up2, int in_cs0, int cout_main, int mode) {
-    TrunkLayer t;
-    memset(&t, 0, sizeof(t));
-    t.wpacked = wq; t.bias = bias; t.out_bf16 = out; t.out_f32 = out_f32; t.res1 = res1; t.res2 = res2;
-    t.stash_out = nullptr;
-    t.cin = cin; t.cout = cout; t.in_map = in_map; t.in_cs0 = in_cs0; t.act = act; t.up2 = up2;
-    t.out_cs_total = out_cs_total; t.out_cs0 = out_cs0; t.cout_main = cout_main; t.res1_cs_total = 16;
-    t.beta = beta; t.mode = mode;
-    T.push_back(t);
-  };
   const int ic = g->inter, cc = 64 + 4 * ic, ccs = cc / 8;
   __nv_bfloat16* cat[2] = {bf(L.cat[0]), bf(L.cat[1])};
   float* a1 = f32(L.a1);
   float* fb[3] = {f32(L.f32[0]), f32(L.f32[1]), f32(L.f32[2])};
-  layer(image("pre"), P(g, "pre_residual_conv_layer/b"), 128, 64, 0, 1, 0.f, cat[0], ccs, 0, a1, nullptr, nullptr, 0, 0,
-        64, 0);
+  add_pass(T, a.image("pre"), P(g, "pre_residual_conv_layer/b"), 128, 64, 0, 1, 0.f, cat[0], ccs, 0, a1, nullptr,
+           nullptr, 0, 0, 64, 0);
   int cur = 0, fi = 0;
   float* cur_f32 = a1;
   for (int i = 0; i < g->nb; ++i) {
@@ -288,90 +324,39 @@ static void build_trunk_table(Gen* g, const WsLayout& L, uint8_t* ws) {
       if (L.paired) {
         for (int k = 1; k <= 3; k += 2) {
           const int cin = 64 + (k - 1) * ic;
-          layer(image(pre + "/pair" + std::to_string(k)), bias(k), cin, 64, 1 + cur, 1, 0.f, cat[cur], ccs, cin / 8,
-                nullptr, nullptr, nullptr, 0, 0, 32, 1);
-          layer(image(pre + "/tail" + std::to_string(k + 1)), bias(k + 1), 32, 32, 1 + cur, 1, 0.f, cat[cur], ccs,
-                cin / 8 + 4, nullptr, nullptr, nullptr, 0, cin / 8, 32, 2);
+          add_pass(T, a.image(pre + "/pair" + std::to_string(k)), bias(k), cin, 64, 1 + cur, 1, 0.f, cat[cur], ccs,
+                   cin / 8, nullptr, nullptr, nullptr, 0, 0, 32, 1);
+          add_pass(T, a.image(pre + "/tail" + std::to_string(k + 1)), bias(k + 1), 32, 32, 1 + cur, 1, 0.f, cat[cur],
+                   ccs, cin / 8 + 4, nullptr, nullptr, nullptr, 0, cin / 8, 32, 2);
         }
       } else {
         for (int k = 1; k <= 4; ++k) {
           const int cin = 64 + (k - 1) * ic;
-          layer(image(pre + "/c" + std::to_string(k)), bias(k), cin, ic, 1 + cur, 1, 0.f, cat[cur], ccs, cin / 8, nullptr,
-                nullptr, nullptr, 0, 0, ic, 0);
+          add_pass(T, a.image(pre + "/c" + std::to_string(k)), bias(k), cin, ic, 1 + cur, 1, 0.f, cat[cur], ccs, cin / 8,
+                   nullptr, nullptr, nullptr, 0, 0, ic, 0);
         }
       }
       while (fb[fi] == cur_f32 || fb[fi] == rrdb_in) fi = (fi + 1) % 3;
       float* nxt = fb[fi];
-      layer(image(pre + "/c5"), bias(5), cc, 64, 1 + cur, 0, g->beta, cat[1 - cur], ccs, 0, nxt, cur_f32,
-            r == 3 ? rrdb_in : nullptr, 0, 0, 64, 0);
+      add_pass(T, a.image(pre + "/c5"), bias(5), cc, 64, 1 + cur, 0, g->beta, cat[1 - cur], ccs, 0, nxt, cur_f32,
+               r == 3 ? rrdb_in : nullptr, 0, 0, 64, 0);
       cur = 1 - cur;
       cur_f32 = nxt;
     }
   }
-  layer(image("post"), P(g, "post_residual_conv_layer/b"), 64, 64, 1 + cur, 0, 1.f, bf(L.u1), 8, 0, nullptr, a1, nullptr,
-        1, 0, 64, 0);
+  add_pass(T, a.image("post"), P(g, "post_residual_conv_layer/b"), 64, 64, 1 + cur, 0, 1.f, bf(L.u1), 8, 0, nullptr, a1,
+           nullptr, 1, 0, 64, 0);
 }
 
 // ---- precision "bf16x3": split-bf16 operand images, workspace and pass tables ---------------------------------------
 // (the C++ twin of model.py's _pack("split") / _split_workspace / _forward_split)
 static int build_split_pack_plan(Gen* g) {
-  if (g->arena_s) return DBM_OK;
-  std::vector<PackEntry> ent;
-  size_t off = 0;
-  auto image = [&](const std::string& name, int cin, int coutp) {
-    g->img_s[name] = off;
-    off += ((size_t)3 * 9 * cin * coutp * 2 + 255) & ~(size_t)255;
-    return g->img_s[name];
-  };
-  auto entry = [&](const std::string& wkey, size_t img_off, int O, int o0, int cin, int cin_total, int c0, int coutp) {
-    PackEntry e;
-    e.w = P(g, wkey);
-    e.out = (__nv_bfloat16*)img_off;
-    e.O = O; e.o0 = o0; e.Cin = cin; e.CinTotal = cin_total; e.c0 = c0; e.COUTP = coutp; e.CK = 16; e.mode = 16;
-    ent.push_back(e);
-  };
-  const int ic = g->inter, cc = 64 + 4 * ic;
-  entry("pre_residual_conv_layer/W", image("pre", 128, 64), 64, 0, 128, 128, 0, 64);
-  for (int i = 0; i < g->nb; ++i)
-    for (int r = 1; r <= 3; ++r) {
-      const std::string pre = rdb_prefix(i, r);
-      entry(pre + "/conv_layer5/W", image(pre + "/c5", cc, 64), 64, 0, cc, cc, 0, 64);
-      if (ic == 32) {
-        for (int k = 1; k <= 3; k += 2) {
-          const int cin = 64 + (k - 1) * 32;
-          const std::string wa = pre + "/conv_layer" + std::to_string(k) + "/W";
-          const std::string wb = pre + "/conv_layer" + std::to_string(k + 1) + "/W";
-          const size_t both = image(pre + "/pair" + std::to_string(k), cin, 64);
-          entry(wa, both, 32, 0, cin, cin, 0, 64);
-          entry(wb, both, 32, 32, cin, cin + 32, 0, 64);
-          entry(wb, image(pre + "/tail" + std::to_string(k + 1), 32, 32), 32, 0, 32, cin + 32, cin, 32);
-        }
-      } else {
-        for (int k = 1; k <= 4; ++k) {
-          const int cin = 64 + (k - 1) * ic;
-          entry(pre + "/conv_layer" + std::to_string(k) + "/W", image(pre + "/c" + std::to_string(k), cin, ic), ic, 0, cin,
-                cin, 0, ic);
-        }
-      }
-    }
-  entry("post_residual_conv_layer/W", image("post", 64, 64), 64, 0, 64, 64, 0, 64);
-  entry("post_upsample_conv_layer_1/W", image("up1", 64, 64), 64, 0, 64, 64, 0, 64);
-  entry("post_upsample_conv_layer_2/W", image("up2", 64, 64), 64, 0, 64, 64, 0, 64);
-  g->arena_s_bytes = off;
-  DBM_CUDA(cudaMalloc(&g->arena_s, off));
-  DBM_CUDA(cudaMemset(g->arena_s, 0, off));
-  long mx = 0;
-  for (auto& e : ent) {
-    e.out = (__nv_bfloat16*)(g->arena_s + (size_t)e.out);
-    const long el = (long)9 * e.Cin * e.COUTP;
-    if (el > mx) mx = el;
-  }
-  g->pack_s_n = (int)ent.size();
-  g->pack_s_max = mx;
-  DBM_CUDA(cudaMalloc(&g->pack_s_dev, ent.size() * sizeof(PackEntry)));
-  DBM_CUDA(cudaMemcpy(g->pack_s_dev, ent.data(), ent.size() * sizeof(PackEntry), cudaMemcpyHostToDevice));
-  g->stale_s = true;
-  return DBM_OK;
+  if (g->pack_s.base) return DBM_OK;
+  PackPlan p{g, g->pack_s, 3, 16};
+  trunk_pack_entries(p, g->inter != 32);   // inter_channels 32: the paired images only
+  p.entry("post_upsample_conv_layer_1/W", p.image("up1", 64, 64), 64, 0, 64, 64, 0, 64, 16);
+  p.entry("post_upsample_conv_layer_2/W", p.image("up2", 64, 64), 64, 0, 64, 64, 0, 64, 16);
+  return upload(p);
 }
 
 struct WsSplit {
@@ -421,68 +406,16 @@ static WsSplit ws_layout_split(const Gen* g, int n, int h, int w) {
   return L;
 }
 
-// Pass tables of the split path: the trunk's (same passes as the bf16 table; cs fields stay logical) followed by the
-// two single-pass tables of the upsample convs
+// Pass tables of the split path: the trunk's (same passes as the bf16 table) followed by the two single-pass tables of
+// the upsample convs
 static int build_split_tables(Gen* g, const WsSplit& L, uint8_t* ws, std::vector<TrunkLayer>& T) {
-  T.clear();
-  auto bf = [&](size_t o) { return (__nv_bfloat16*)(ws + o); };
-  auto f32 = [&](size_t o) { return (float*)(ws + o); };
-  auto image = [&](const std::string& name) { return (const __nv_bfloat16*)(g->arena_s + g->img_s.at(name)); };
-  auto layer = [&](const __nv_bfloat16* wq, const float* bias, int cin, int cout, int in_map, int act, float beta,
-                   __nv_bfloat16* out, int out_cs_total, int out_cs0, float* out_f32, const float* res1,
-                   const float* res2, int up2, int in_cs0, int cout_main, int mode) {
-    TrunkLayer t;
-    memset(&t, 0, sizeof(t));
-    t.wpacked = wq; t.bias = bias; t.out_bf16 = out; t.out_f32 = out_f32; t.res1 = res1; t.res2 = res2;
-    t.cin = cin; t.cout = cout; t.in_map = in_map; t.in_cs0 = in_cs0; t.act = act; t.up2 = up2;
-    t.out_cs_total = out_cs_total; t.out_cs0 = out_cs0; t.cout_main = cout_main; t.res1_cs_total = 16;
-    t.beta = beta; t.mode = mode;
-    T.push_back(t);
-  };
-  const int ic = g->inter, cc = 64 + 4 * ic, ccs = cc / 8;
-  DBM_REQUIRE(L.paired || ic != 32, "gen_forward (bf16x3): tiles wider than ~2000 px are not supported");
-  __nv_bfloat16* cat[2] = {bf(L.cat[0]), bf(L.cat[1])};
-  float* a1 = f32(L.a1);
-  float* fb[3] = {f32(L.f32[0]), f32(L.f32[1]), f32(L.f32[2])};
-  layer(image("pre"), P(g, "pre_residual_conv_layer/b"), 128, 64, 0, 1, 0.f, cat[0], ccs, 0, a1, nullptr, nullptr, 0, 0,
-        64, 0);
-  int cur = 0, fi = 0;
-  float* cur_f32 = a1;
-  for (int i = 0; i < g->nb; ++i) {
-    float* rrdb_in = cur_f32;
-    for (int r = 1; r <= 3; ++r) {
-      const std::string pre = rdb_prefix(i, r);
-      auto bias = [&](int k) { return P(g, pre + "/conv_layer" + std::to_string(k) + "/b"); };
-      if (ic == 32) {
-        for (int k = 1; k <= 3; k += 2) {
-          const int cin = 64 + (k - 1) * ic;
-          layer(image(pre + "/pair" + std::to_string(k)), bias(k), cin, 64, 1 + cur, 1, 0.f, cat[cur], ccs, cin / 8,
-                nullptr, nullptr, nullptr, 0, 0, 32, 1);
-          layer(image(pre + "/tail" + std::to_string(k + 1)), bias(k + 1), 32, 32, 1 + cur, 1, 0.f, cat[cur], ccs,
-                cin / 8 + 4, nullptr, nullptr, nullptr, 0, cin / 8, 32, 2);
-        }
-      } else {
-        for (int k = 1; k <= 4; ++k) {
-          const int cin = 64 + (k - 1) * ic;
-          layer(image(pre + "/c" + std::to_string(k)), bias(k), cin, ic, 1 + cur, 1, 0.f, cat[cur], ccs, cin / 8, nullptr,
-                nullptr, nullptr, 0, 0, ic, 0);
-        }
-      }
-      while (fb[fi] == cur_f32 || fb[fi] == rrdb_in) fi = (fi + 1) % 3;
-      float* nxt = fb[fi];
-      layer(image(pre + "/c5"), bias(5), cc, 64, 1 + cur, 0, g->beta, cat[1 - cur], ccs, 0, nxt, cur_f32,
-            r == 3 ? rrdb_in : nullptr, 0, 0, 64, 0);
-      cur = 1 - cur;
-      cur_f32 = nxt;
-    }
-  }
-  layer(image("post"), P(g, "post_residual_conv_layer/b"), 64, 64, 1 + cur, 0, 1.f, bf(L.u1), 8, 0, nullptr, a1, nullptr,
-        1, 0, 64, 0);
+  DBM_REQUIRE(L.paired || g->inter != 32, "gen_forward (bf16x3): tiles wider than ~2000 px are not supported");
+  build_trunk_passes(g, g->pack_s, L, ws, T);
   // upsample convs: single-pass tables of the same kernel at 2x / 4x the resolution (input = "stem" map 0)
-  layer(image("up1"), P(g, "post_upsample_conv_layer_1/b"), 64, 64, 0, 1, 0.f, bf(L.u2), 8, 0, nullptr, nullptr, nullptr, 1,
-        0, 64, 0);
-  layer(image("up2"), P(g, "post_upsample_conv_layer_2/b"), 64, 64, 0, 1, 0.f, nullptr, 0, 0, f32(L.c2f), nullptr, nullptr,
-        0, 0, 64, 0);
+  add_pass(T, g->pack_s.image("up1"), P(g, "post_upsample_conv_layer_1/b"), 64, 64, 0, 1, 0.f,
+           (__nv_bfloat16*)(ws + L.u2), 8, 0, nullptr, nullptr, nullptr, 1, 0, 64, 0);
+  add_pass(T, g->pack_s.image("up2"), P(g, "post_upsample_conv_layer_2/b"), 64, 64, 0, 1, 0.f, nullptr, 0, 0,
+           (float*)(ws + L.c2f), nullptr, nullptr, 0, 0, 64, 0);
   return DBM_OK;
 }
 
@@ -495,10 +428,7 @@ static int gen_forward_split(Gen* g, const float* x, const float* w1, const floa
               workspace_bytes, L.total);
   uint8_t* ws = (uint8_t*)workspace;
   const int H = h_in - 2, W = w_in - 2;
-  if (g->stale_s) {
-    if ((rc = dbm_pack_conv3x3_table(g->pack_s_dev, g->pack_s_n, g->pack_s_max, st))) return rc;
-    g->stale_s = false;
-  }
+  if ((rc = refresh(g->pack_s, st))) return rc;
   if (g->tab_ws != workspace || g->tab_n != n || g->tab_h != h_in || g->tab_w != w_in || g->tab_precision != 1) {
     if ((rc = build_split_tables(g, L, ws, g->tab_host))) return rc;
     DBM_REQUIRE((int)g->tab_host.size() == L.num_layers + 2, "gen_forward: split pass tables have %zu entries, expected %d",
@@ -604,10 +534,8 @@ extern "C" int dbm_gen_destroy(dbm_gen* h) {
   if (!h) return DBM_OK;
   Gen* g = &h->g;
   if (g->owns_flat && g->flat) cudaFree(g->flat);
-  if (g->arena) cudaFree(g->arena);
-  if (g->pack_dev) cudaFree(g->pack_dev);
-  if (g->arena_s) cudaFree(g->arena_s);
-  if (g->pack_s_dev) cudaFree(g->pack_s_dev);
+  free_arena(g->pack);
+  free_arena(g->pack_s);
   delete h;
   return DBM_OK;
 }
@@ -638,8 +566,7 @@ extern "C" int dbm_gen_set_param(dbm_gen* h, const char* key, const float* host_
   DBM_REQUIRE(ok, "gen_set_param: '%s' has shape (%d,%d,%d,%d), got %d-d (%d,...)", key, p.dims[0], p.dims[1],
               p.dims[2], p.dims[3], ndim, ndim > 0 ? dims[0] : 0);
   DBM_CUDA(cudaMemcpy(g->flat + p.off, host_values, (size_t)p.n * 4, cudaMemcpyHostToDevice));
-  g->stale = true;
-  g->stale_s = true;
+  g->pack.stale = g->pack_s.stale = true;
   return DBM_OK;
 }
 
@@ -650,29 +577,19 @@ extern "C" int dbm_gen_bind_params(dbm_gen* h, float* device_flat) {
   Gen* g = &h->g;
   DBM_REQUIRE(g->owns_flat, "gen_bind_params: parameters are already bound");
   cudaFree(g->flat);
-  // rebase the pack table's filter pointers
-  std::vector<PackEntry> ent(g->pack_n);
-  DBM_CUDA(cudaMemcpy(ent.data(), g->pack_dev, ent.size() * sizeof(PackEntry), cudaMemcpyDeviceToHost));
-  for (auto& e : ent) e.w = device_flat + (e.w - g->flat);
-  DBM_CUDA(cudaMemcpy(g->pack_dev, ent.data(), ent.size() * sizeof(PackEntry), cudaMemcpyHostToDevice));
-  if (g->pack_s_dev) {
-    std::vector<PackEntry> es(g->pack_s_n);
-    DBM_CUDA(cudaMemcpy(es.data(), g->pack_s_dev, es.size() * sizeof(PackEntry), cudaMemcpyDeviceToHost));
-    for (auto& e : es) e.w = device_flat + (e.w - g->flat);
-    DBM_CUDA(cudaMemcpy(g->pack_s_dev, es.data(), es.size() * sizeof(PackEntry), cudaMemcpyHostToDevice));
-  }
+  int rc;
+  if ((rc = rebase_weights(g->pack, g->flat, device_flat)) || (rc = rebase_weights(g->pack_s, g->flat, device_flat)))
+    return rc;
   g->flat = device_flat;
   g->owns_flat = false;
-  g->stale = true;
-  g->stale_s = true;
+  g->pack.stale = g->pack_s.stale = true;
   g->tab_ws = nullptr;
   return DBM_OK;
 }
 
 extern "C" int dbm_gen_mark_updated(dbm_gen* h) {
   DBM_REQUIRE(h != nullptr, "gen_mark_updated: null handle");
-  h->g.stale = true;
-  h->g.stale_s = true;
+  h->g.pack.stale = h->g.pack_s.stale = true;
   return DBM_OK;
 }
 
@@ -712,7 +629,7 @@ extern "C" int dbm_gen_forward(dbm_gen* h, const float* x, const float* w1, cons
   int rc = refresh_packed(g, st);
   if (rc) return rc;
   if (g->tab_ws != workspace || g->tab_n != n || g->tab_h != h_in || g->tab_w != w_in || g->tab_precision != 0) {
-    build_trunk_table(g, L, ws);
+    build_trunk_passes(g, g->pack, L, ws, g->tab_host);
     DBM_REQUIRE((int)g->tab_host.size() == L.num_layers, "gen_forward: pass table has %zu entries, expected %d",
                 g->tab_host.size(), L.num_layers);
     // the table is read by this very stream's kernels only: an ordered copy is enough
@@ -723,13 +640,14 @@ extern "C" int dbm_gen_forward(dbm_gen* h, const float* x, const float* w1, cons
   }
   void* s2d = ws + L.s2d;
   void* s0 = ws + L.s0;
-  const float* wts = (const float*)(g->arena + g->off_wts);
-  const float* bias128 = (const float*)(g->arena + g->off_bias128);
-  auto image = [&](const char* name) { return (const void*)(g->arena + g->img.at(name)); };
+  const uint8_t* arena = g->pack.base;
+  const float* wts = (const float*)(arena + g->off_wts);
+  const float* bias128 = (const float*)(arena + g->off_bias128);
+  auto image = [&](const char* name) { return (const void*)g->pack.image(name); };
   // ---- input block (srgan_train.py:256-266) ----
   if ((rc = dbm_stem_w1_s2d(w1, s2d, n, h_in, w_in, st))) return rc;
   if ((rc = dbm_stem_fwd_slab8(x, nullptr, w2, w3, nullptr, wts, bias128, s0, 16, 0, n, h_in, w_in, st))) return rc;
-  if ((rc = dbm_conv3x3_umma_valid(s2d, 40, 320, g->arena + g->off_w1tc, P(g, "input_block/conv_on_W1/b"), n, h_in, w_in,
+  if ((rc = dbm_conv3x3_umma_valid(s2d, 40, 320, arena + g->off_w1tc, P(g, "input_block/conv_on_W1/b"), n, h_in, w_in,
                                    s0, 16, 4, st)))
     return rc;
   // ---- pre-residual conv, 12 x RRDB, post-residual conv + skip + nearest x2 (:541-558) ----
@@ -749,14 +667,14 @@ extern "C" int dbm_gen_forward(dbm_gen* h, const float* x, const float* w1, cons
                              f1, 8, 0, nullptr, 0, 0, nullptr, nullptr, st)))
     return rc;
   // ---- deformable layers (:572-574) ----
-  if ((rc = dbm_conv3x3_umma(f1, 8, 64, image("off1"), (const float*)(g->arena + g->off_bias_off1), 32, n, 4 * H, 4 * W,
+  if ((rc = dbm_conv3x3_umma(f1, 8, 64, image("off1"), (const float*)(arena + g->off_bias_off1), 32, n, 4 * H, 4 * W,
                              0.f, 0, 0, nullptr, 0, 0, offs, 8, 0, nullptr, nullptr, st)))
     return rc;
   void* d1 = u2;
   if ((rc = dbm_deform_conv_umma(f1, offs, 8, image("dc1"), P(g, "final_conv_layer1/deform_conv/b"), n, 4 * H, 4 * W, 1, d1,
                                  8, 0, nullptr, nullptr, st)))
     return rc;
-  if ((rc = dbm_conv3x3_umma(d1, 8, 64, image("off2"), (const float*)(g->arena + g->off_bias_off2), 32, n, 4 * H, 4 * W,
+  if ((rc = dbm_conv3x3_umma(d1, 8, 64, image("off2"), (const float*)(arena + g->off_bias_off2), 32, n, 4 * H, 4 * W,
                              0.f, 0, 0, nullptr, 0, 0, offs, 8, 0, nullptr, nullptr, st)))
     return rc;
   return dbm_deform_conv_out1(d1, offs, 8, P(g, "final_conv_layer2/deform_conv/W"), P(g, "final_conv_layer2/deform_conv/b"),

@@ -139,6 +139,69 @@ def rdb_plan(nrdb: int, beta: float):
     return plan
 
 
+def epi(**kw):
+    """One FlatEpiBlock record; scales default to 1."""
+    e = np.zeros((), dtype=EPI_DTYPE)
+    e["s1"] = 1.0
+    e["beta"] = 1.0
+    e["beta2"] = 1.0
+    e["out_scale"] = 1.0
+    for k, v in kw.items():
+        e[k] = v
+    return e
+
+
+def launch(inp_ptr, wq, cin, nout, blocks):
+    """One FlatLaunch record: a 3x3 conv of ``cin`` channels at ``inp_ptr`` with packed filter ``wq``, N = ``nout``,
+    one epilogue block per 32 output channels."""
+    L = np.zeros((), dtype=LAUNCH_DTYPE)
+    L["in"] = inp_ptr
+    L["wpacked"] = wq.data_ptr()
+    L["cin"] = cin
+    L["nout"] = nout
+    L["ny"] = 1
+    assert len(blocks) == nout // 32
+    for b, e in enumerate(blocks):
+        L["blk"][b] = e
+    return L
+
+
+def forward_chain(model, pk, Pg, s0, cat, x, a3f):
+    """Launch records of the trunk's forward (srgan_train.py:541-551) on the flat-padded layout, ``Pg`` positions per
+    channel: the pre-residual conv from the stem output ``s0``, the 3 * nb residual dense blocks, the post-residual conv
+    with the skip a1 into ``a3f``. Dense block j reads [a0 | a1..a4] from ``cat(j)`` (filling a1..a4 there) and writes
+    its bf16 output into ``cat(j + 1)``; ``x(j)`` is the fp32 residual stream into block j (``x(0)`` = a1)."""
+    beta, g = model.residual_scaling, model.inter_channels
+    pb = lambda t, c=0: t.data_ptr() + 2 * c * Pg
+    pf = lambda t, c=0: t.data_ptr() + 4 * c * Pg
+    nrdb = 3 * model.num_residual_blocks
+    wq, bq = pk["pre_residual_conv_layer@trunk"]
+    tab = [launch(pb(s0), wq, 128, 64, [
+        epi(bias=bq.data_ptr() + 128 * b, act=1, out_f32=pf(x(0), 32 * b), out_bf16=pb(cat(0), 32 * b)) for b in range(2)])]
+    for j in range(nrdb):
+        r = j % 3 + 1
+        pre = model._rdb_prefix(j // 3, r)
+        for k in (1, 2, 3, 4):
+            cin = 64 + g * (k - 1)
+            wq, bq = pk[f"{pre}/conv_layer{k}@trunk"]
+            tab.append(launch(pb(cat(j)), wq, cin, g, [
+                epi(bias=bq.data_ptr() + 128 * b, act=1, out_bf16=pb(cat(j), cin + 32 * b)) for b in range(g // 32)]))
+        wq, bq = pk[f"{pre}/conv_layer5@trunk"]
+        blocks = []
+        for b in range(2):
+            kw = dict(bias=bq.data_ptr() + 128 * b, add1=pf(x(j), 32 * b), s1=1.0, beta=beta,
+                      out_f32=pf(x(j + 1), 32 * b), out_bf16=pb(cat(j + 1), 32 * b))
+            if r == 3:   # out = rrdb_in + beta * (x + beta * a5)  (srgan_train.py:358, 402)
+                kw.update(add2=pf(x(j - 2), 32 * b), beta2=beta)
+            blocks.append(epi(**kw))
+        tab.append(launch(pb(cat(j)), wq, 64 + 4 * g, 64, blocks))
+    wq, bq = pk["post_residual_conv_layer@trunk"]
+    tab.append(launch(pb(cat(nrdb)), wq, 64, 64, [
+        epi(bias=bq.data_ptr() + 128 * b, add1=pf(x(0), 32 * b), s1=1.0, beta=1.0, out_f32=pf(a3f, 32 * b))
+        for b in range(2)]))
+    return tab
+
+
 class FlatTrunk:
     """Buffers + tables of the tensor-core training trunk for one (batch, H, W)."""
 
@@ -183,36 +246,13 @@ class FlatTrunk:
     def _x(self, j):
         return self.x0 if j == 0 else self.xring[j % 4]
 
-    @staticmethod
-    def _epi(**kw):
-        e = np.zeros((), dtype=EPI_DTYPE)
-        e["s1"] = 1.0
-        e["beta"] = 1.0
-        e["beta2"] = 1.0
-        e["out_scale"] = 1.0
-        for k, v in kw.items():
-            e[k] = v
-        return e
-
     def _launches(self, inp_ptr, slices, cin, blocks):
         """One conv whose N exceeds the kernels' 192 columns as consecutive launches over N-slices of its operand
         (``slices``: [(n0, width, packed image)], model._pack's ``@dgrad_slices``); ``blocks`` cover all of N."""
         out = []
         for n0, width, img in slices:
-            out.append(self._launch(inp_ptr, img, cin, width, blocks[n0 // 32:(n0 + width) // 32]))
+            out.append(launch(inp_ptr, img, cin, width, blocks[n0 // 32:(n0 + width) // 32]))
         return out
-
-    def _launch(self, inp_ptr, wq, cin, nout, blocks):
-        L = np.zeros((), dtype=LAUNCH_DTYPE)
-        L["in"] = inp_ptr
-        L["wpacked"] = wq.data_ptr()
-        L["cin"] = cin
-        L["nout"] = nout
-        L["ny"] = 1
-        assert len(blocks) == nout // 32
-        for b, e in enumerate(blocks):
-            L["blk"][b] = e
-        return L
 
     def build(self, pk):
         """(Re)build every table against the model's packed-operand buffers ``pk`` (model._pack())."""
@@ -223,45 +263,19 @@ class FlatTrunk:
         P, Gr = m.p, m.g
         G, cc = self.G, self.cc
         nrdb = self.nrdb
-        pb, pf, epi = self._pb, self._pf, self._epi
+        pb, pf = self._pb, self._pf
         plan = rdb_plan(nrdb, beta)
-        fwd, bwd = [], []
+        bwd = []
         convs = []  # (key, act tensor, cin, g tensor, g channel0, cout) for the weight / bias gradients
 
-        # ---------------- forward chain ----------------
-        wq, bq = pk["pre_residual_conv_layer@trunk"]
-        fwd.append(self._launch(pb(self.s0), wq, 128, 64, [
-            epi(bias=bq.data_ptr() + 128 * b, act=1, out_f32=pf(self.x0, 32 * b), out_bf16=pb(self.cat[0], 32 * b))
-            for b in range(2)]))
-        for d in plan:
-            j, r = d["j"], d["r"]
-            pre = m._rdb_prefix(j // 3, r)
-            cat = self.cat[j]
-            for k in (1, 2, 3, 4):
-                cin = 64 + G * (k - 1)
-                wq, bq = pk[f"{pre}/conv_layer{k}@trunk"]
-                fwd.append(self._launch(pb(cat), wq, cin, G, [
-                    epi(bias=bq.data_ptr() + 128 * b, act=1, out_bf16=pb(cat, cin + 32 * b)) for b in range(G // 32)]))
-            wq, bq = pk[f"{pre}/conv_layer5@trunk"]
-            blocks = []
-            for b in range(2):
-                kw = dict(bias=bq.data_ptr() + 128 * b, add1=pf(self._x(j), 32 * b), s1=1.0, beta=beta,
-                          out_f32=pf(self._x(j + 1), 32 * b), out_bf16=pb(self.cat[j + 1], 32 * b))
-                if r == 3:
-                    kw.update(add2=pf(self._x(j - 2), 32 * b), beta2=beta)
-                blocks.append(epi(**kw))
-            fwd.append(self._launch(pb(cat), wq, cc, 64, blocks))
-        wq, bq = pk["post_residual_conv_layer@trunk"]
-        fwd.append(self._launch(pb(self.cat[nrdb]), wq, 64, 64, [
-            epi(bias=bq.data_ptr() + 128 * b, add1=pf(self.x0, 32 * b), s1=1.0, beta=1.0, out_f32=pf(self.a3f, 32 * b))
-            for b in range(2)]))
+        fwd = forward_chain(m, pk, self.Pg, self.s0, lambda j: self.cat[j], self._x, self.a3f)
 
         # ---------------- data-gradient chain ----------------
         dX = lambda j: self.dX[j % 4]
         gb = G // 32                       # 32-channel epilogue blocks per dense-block slot
         nb5 = cc // 32                     # blocks of conv5's data gradient d[a0 .. a4]
         wq = pk["post_residual_conv_layer@dgrad"]
-        bwd.append(self._launch(pb(self.gpost), wq, 64, 64, [
+        bwd.append(launch(pb(self.gpost), wq, 64, 64, [
             epi(out_f32=pf(dX(nrdb), 32 * b), out_bf16=pb(self.gcat[nrdb - 1], 4 * G + 32 * b),
                 out_scale=plan[nrdb - 1]["g5_scale"]) for b in range(2)]))
         convs.append(("post_residual_conv_layer", self.cat[nrdb], 64, self.gpost, 0, 64))
@@ -308,10 +322,10 @@ class FlatTrunk:
                 else:   # a1 = lrelu(pre_res(a0)) (:541-544)
                     kw.update(mask=pb(self.cat[0], 32 * b), out_bf16=pb(self.gpre, 32 * b))
                 blocks.append(epi(**kw))
-            bwd.append(self._launch(pb(gcat, 0), pk[f"{pre}/conv_layer1@dgrad"], G, 64, blocks))
+            bwd.append(launch(pb(gcat, 0), pk[f"{pre}/conv_layer1@dgrad"], G, 64, blocks))
             convs.append((f"{pre}/conv_layer1", cat, 64, gcat, 0, G))
-        bwd.append(self._launch(pb(self.gpre), pk["pre_residual_conv_layer@dgrad"], 64, 128,
-                                [epi(out_f32=pf(self.da0f, 32 * b)) for b in range(4)]))
+        bwd.append(launch(pb(self.gpre), pk["pre_residual_conv_layer@dgrad"], 64, 128,
+                          [epi(out_f32=pf(self.da0f, 32 * b)) for b in range(4)]))
         convs.append(("pre_residual_conv_layer", self.s0, 128, self.gpre, 0, 64))
 
         # ---------------- weight / bias gradient tables ----------------
@@ -468,38 +482,7 @@ class FlatChainForward:
         key = (m._pack_gen, m.residual_scaling)
         if self._key == key:
             return
-        beta, g, Pg = m.residual_scaling, m.inter_channels, self.Pg
-        pb = lambda t, c=0: t.data_ptr() + 2 * c * Pg
-        pf = lambda t, c=0: t.data_ptr() + 4 * c * Pg
-        epi, launch = FlatTrunk._epi, FlatTrunk._launch
-        nrdb = 3 * m.num_residual_blocks
-        tab = []
-        wq, bq = pk["pre_residual_conv_layer@trunk"]
-        tab.append(launch(self, pb(self.s0), wq, 128, 64, [
-            epi(bias=bq.data_ptr() + 128 * b, act=1, out_f32=pf(self.x0, 32 * b), out_bf16=pb(self.cat[0], 32 * b))
-            for b in range(2)]))
-        for j in range(nrdb):
-            r = j % 3 + 1
-            pre = m._rdb_prefix(j // 3, r)
-            cat, nxt = self.cat[j % 2], self.cat[(j + 1) % 2]
-            for k in (1, 2, 3, 4):
-                cin = 64 + g * (k - 1)
-                wq, bq = pk[f"{pre}/conv_layer{k}@trunk"]
-                tab.append(launch(self, pb(cat), wq, cin, g, [
-                    epi(bias=bq.data_ptr() + 128 * b, act=1, out_bf16=pb(cat, cin + 32 * b)) for b in range(g // 32)]))
-            wq, bq = pk[f"{pre}/conv_layer5@trunk"]
-            blocks = []
-            for b in range(2):
-                kw = dict(bias=bq.data_ptr() + 128 * b, add1=pf(self._x(j), 32 * b), s1=1.0, beta=beta,
-                          out_f32=pf(self._x(j + 1), 32 * b), out_bf16=pb(nxt, 32 * b))
-                if r == 3:   # out = rrdb_in + beta * (x + beta * a5)  (srgan_train.py:358, 402)
-                    kw.update(add2=pf(self._x(j - 2), 32 * b), beta2=beta)
-                blocks.append(epi(**kw))
-            tab.append(launch(self, pb(cat), wq, self.cc, 64, blocks))
-        wq, bq = pk["post_residual_conv_layer@trunk"]
-        tab.append(launch(self, pb(self.cat[nrdb % 2]), wq, 64, 64, [
-            epi(bias=bq.data_ptr() + 128 * b, add1=pf(self.x0, 32 * b), s1=1.0, beta=1.0, out_f32=pf(self.a3f, 32 * b))
-            for b in range(2)]))
+        tab = forward_chain(m, pk, self.Pg, self.s0, lambda j: self.cat[j % 2], self._x, self.a3f)
         self.table = np.ascontiguousarray(np.stack(tab))
         self.table_dev = torch.from_numpy(self.table.view(np.uint8).reshape(-1).copy()).cuda()
         self.flags = ops.empty(len(tab) * self.geom["tiles"], dtype=torch.int32)
@@ -563,7 +546,7 @@ def conv3x3(inp: torch.Tensor, cin: int, wpacked: torch.Tensor, nout: int, block
     L[0]["nout"] = nout
     L[0]["ny"] = 1
     for b, kw in enumerate(blocks):
-        L[0]["blk"][b] = FlatTrunk._epi(**kw)
+        L[0]["blk"][b] = epi(**kw)
     ops.call("dbm_flat_conv3x3_seq", L.ctypes.data, 1, n, h, w, 0, 0, ops.stream())
 
 
@@ -654,7 +637,6 @@ class FlatConv:
         self.zf = alloc_f32(im.Opad, self.geom)
         self.gin = alloc_bf16(im.Opad, self.geom)
         self.dxf = alloc_f32(im.Cg, self.geom)
-        epi = FlatTrunk._epi
         self.rec_f = []
         for slot in range(nslots):
             L = np.zeros(1, dtype=LAUNCH_DTYPE)

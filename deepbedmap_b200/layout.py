@@ -1,6 +1,6 @@
 """Parameter inventory of the generator / discriminator in the reference's Chainer ``.npz`` key
 layout (chainer.serializers.save_npz of the links defined at srgan_train.py:201-699; call sites
-srgan_train.py:1355-1361, deepbedmap.py:408)."""
+srgan_train.py:1355-1361, deepbedmap.py:408), and the generator trunk's pass plan (trunk_plan)."""
 from __future__ import annotations
 
 import math
@@ -85,6 +85,63 @@ def init_values(shapes, seed: int, scale: float = 0.1):
         else:
             out[k] = np.zeros(shp, np.float32)
     return out
+
+
+def trunk_pass(image, cin, cout, in_map, bias=None, act=0, beta=0.0, out=None, out_cs0=0, out_f32=None, res1=None,
+               res2=None, up2=0, in_cs0=0, cout_main=None, mode=0):
+    """One pass of the trunk kernels (csrc/umma_trunk.cu TrunkLayer) with symbolic operands: ``image`` names the packed
+    filter image (model._pack's key without its @trunk / @split suffix), ``bias`` the bias key (default ``image/b``);
+    ``in_map`` 0 reads the stem output, 1 / 2 the dense-block buffers cat0 / cat1; ``out`` names the bf16 output buffer
+    ("cat0", "cat1", "u1", ...) and ``out_f32`` / ``res1`` / ``res2`` the fp32 ones ("a1", "f32_0".."f32_2")."""
+    return dict(image=image, bias=f"{image}/b" if bias is None else bias, cin=cin, cout=cout, in_map=in_map,
+                in_cs0=in_cs0, act=act, up2=up2, out=out, out_cs0=out_cs0,
+                cout_main=cout if cout_main is None else cout_main, beta=beta, mode=mode, out_f32=out_f32, res1=res1,
+                res2=res2)
+
+
+def trunk_plan(num_residual_blocks: int, inter_channels: int, residual_scaling: float, paired: bool,
+               paired_convs=(1, 3)):
+    """Pass sequence of the generator trunk (srgan_train.py:541-558) as trunk_pass records: the pre-residual conv
+    (a1 = lrelu(conv(a0)), kept in fp32), 3 * nb residual dense blocks, then the post-residual conv with the skip a1 and
+    the nearest x2 fused (into u1). Dense block j reads and extends cat[j % 2] and writes its output into the other
+    buffer; the fp32 residual stream rotates through a ring of three buffers so that a conv5 never writes the block
+    input (res1) or, on the third block of an RRDB, the RRDB input (res2) it reads.
+
+    ``paired`` (inter_channels 32 only) fuses conv_k with conv_{k+1} for each k in ``paired_convs`` (1 and / or 3):
+      head ("{pre}/pair{k}", mode 1): N = 64 over [a0..a_{k-1}] -> a_k (32 columns, fused epilogue); the other 32
+          columns -- the partial sums of conv_{k+1} over the same inputs -- stay in tensor memory
+      tail ("{pre}/tail{k+1}", mode 2): N = 32 over a_k only, accumulated onto those columns -> a_{k+1}
+    Same FLOPs; 252 N=32 MMAs per 128-pixel tile become 108 N=64 + 36 N=32 MMAs (each MMA re-reads its 4 KB A operand
+    from shared memory whatever N is), and nothing but the bf16 features a_k ever leaves the SM. A pair not listed is
+    two plain passes."""
+    g = inter_channels
+    ring = ("f32_0", "f32_1", "f32_2")
+    plan = [trunk_pass("pre_residual_conv_layer", 128, 64, 0, act=1, out="cat0", out_f32="a1")]
+    cur, cur_f32, fi = 0, "a1", 0
+    for i in range(num_residual_blocks):
+        rrdb_in = cur_f32
+        for r in (1, 2, 3):
+            pre = f"residual_network/{i}/residual_dense_block{r}"
+            cat = f"cat{cur}"
+            for k in (1, 3):
+                cin = 64 + (k - 1) * g
+                if paired and k in paired_convs:
+                    plan.append(trunk_pass(f"{pre}/pair{k}", cin, 64, 1 + cur, bias=f"{pre}/conv_layer{k}/b", act=1,
+                                           out=cat, out_cs0=cin // 8, cout_main=32, mode=1))
+                    plan.append(trunk_pass(f"{pre}/tail{k + 1}", 32, 32, 1 + cur, bias=f"{pre}/conv_layer{k + 1}/b",
+                                           in_cs0=cin // 8, act=1, out=cat, out_cs0=cin // 8 + 4, mode=2))
+                else:
+                    for kk in (k, k + 1):
+                        ci = 64 + (kk - 1) * g
+                        plan.append(trunk_pass(f"{pre}/conv_layer{kk}", ci, g, 1 + cur, act=1, out=cat, out_cs0=ci // 8))
+            while ring[fi] in (cur_f32, rrdb_in):
+                fi = (fi + 1) % 3
+            plan.append(trunk_pass(f"{pre}/conv_layer5", 64 + 4 * g, 64, 1 + cur, beta=residual_scaling,
+                                   out=f"cat{1 - cur}", out_f32=ring[fi], res1=cur_f32,
+                                   res2=rrdb_in if r == 3 else None))
+            cur, cur_f32 = 1 - cur, ring[fi]
+    plan.append(trunk_pass("post_residual_conv_layer", 64, 64, 1 + cur, beta=1.0, out="u1", res1="a1", up2=1))
+    return plan
 
 
 def infer_num_residual_blocks(keys) -> int:

@@ -610,6 +610,26 @@ class GeneratorModel(_Link):
                             pk[key + "@dgrad"] = slices[0][2]
                         pk[key + "@dgrad_slices"] = slices
 
+            def add_sliced(grp, name, slices, cin, coutp, bias, elems=1, mode=0):
+                # one image assembled from filter slices (wkey, O, o0, cin_total, c0); elems = 3 for split-bf16
+                img = ops.zeros(elems * 9 * cin * coutp, dtype=torch.bfloat16)
+                for wkey, o, o0, cin_total, c0 in slices:
+                    entry(grp, P[wkey], img, o, o0, cin, cin_total, c0, coutp, 16, mode)
+                pk[name] = (img, P[bias])
+
+            def pair_images(pre):
+                # dense-block pairing (layout.trunk_plan, inter_channels = 32): the head image pair{k} holds conv_k and
+                # the rows of conv_{k+1} over their shared inputs (one 64-wide MMA pass), the tail image tail{k+1}
+                # conv_{k+1}'s rows over a_k. (name, slices, cin, coutp, bias key) per image.
+                out = []
+                for k in (1, 3):
+                    cin = 64 + (k - 1) * 32
+                    wa, wb = f"{pre}/conv_layer{k}/W", f"{pre}/conv_layer{k + 1}/W"
+                    out.append((f"{pre}/pair{k}", [(wa, 32, 0, cin, 0), (wb, 32, 32, cin + 32, 0)], cin, 64,
+                                f"{pre}/conv_layer{k}/b"))
+                    out.append((f"{pre}/tail{k + 1}", [(wb, 32, 0, cin + 32, cin)], 32, 32, f"{pre}/conv_layer{k + 1}/b"))
+                return out
+
             add("pre_residual_conv_layer", 64, trunk="io")
             for i in range(self.num_residual_blocks):
                 for r in (1, 2, 3):
@@ -619,21 +639,10 @@ class GeneratorModel(_Link):
                     add(f"{pre}/conv_layer5", 64, trunk="trunk16")
             add("post_residual_conv_layer", 64, trunk="io")
             if self.inter_channels == 32:
-                # dense-block pairing (see _trunk_workspace): conv_k and the partial sums of conv_{k+1}
-                # over their shared inputs are one 64-wide MMA pass; conv_{k+1} then only contracts a_k
                 for i in range(self.num_residual_blocks):
                     for r in (1, 2, 3):
-                        pre = self._rdb_prefix(i, r)
-                        for k in (1, 3):
-                            cin = 64 + (k - 1) * 32
-                            wa, wb = P[f"{pre}/conv_layer{k}/W"], P[f"{pre}/conv_layer{k + 1}/W"]
-                            both = image(cin, 64)
-                            entry("infer", wa, both, 32, 0, cin, cin, 0, 64, 16)
-                            entry("infer", wb, both, 32, 32, cin, cin + 32, 0, 64, 16)
-                            pk[f"{pre}/pair{k}"] = (both, P[f"{pre}/conv_layer{k}/b"])
-                            tail = image(32, 32)
-                            entry("infer", wb, tail, 32, 0, 32, cin + 32, cin, 32, 16)
-                            pk[f"{pre}/tail{k + 1}"] = (tail, P[f"{pre}/conv_layer{k + 1}/b"])
+                        for name, slices, cin, coutp, bias in pair_images(self._rdb_prefix(i, r)):
+                            add_sliced("infer", name, slices, cin, coutp, bias)
                 # input-stationary slices for the image-resident small-tile trunk (csrc/umma_local.cu): pass s
                 # contracts block a_s (a0 = 64 channels, a1..a4 = 32) against its rows in conv_{s+1}..conv_5
                 # stacked along N = 192 - 32 s
@@ -652,34 +661,26 @@ class GeneratorModel(_Link):
                 # split-bf16 operand images (dbm_trunk_umma_split): per 16-channel chunk [w_hi | w_hi | w_lo], 3x the
                 # size of a bf16 image; the trunk's passes (paired plan for inter_channels = 32) and the upsample convs
                 def add_split(name, slices, cin, coutp, bias):
-                    img = ops.zeros(3 * 9 * cin * coutp, dtype=torch.bfloat16)
-                    for wkey, o, o0, cin_total, c0 in slices:
-                        entry("split", P[wkey], img, o, o0, cin, cin_total, c0, coutp, 16, mode=16)
-                    pk[name + "@split"] = (img, bias)
+                    add_sliced("split", name + "@split", slices, cin, coutp, bias, elems=3, mode=16)
 
                 g_ = self.inter_channels
                 for key in ("pre_residual_conv_layer", "post_residual_conv_layer", "post_upsample_conv_layer_1",
                             "post_upsample_conv_layer_2"):
                     w = P[f"{key}/W"]
-                    add_split(key, [(f"{key}/W", w.shape[0], 0, w.shape[1], 0)], w.shape[1], 64, P[f"{key}/b"])
+                    add_split(key, [(f"{key}/W", w.shape[0], 0, w.shape[1], 0)], w.shape[1], 64, f"{key}/b")
                 for i in range(self.num_residual_blocks):
                     for r in (1, 2, 3):
                         pre = self._rdb_prefix(i, r)
                         add_split(f"{pre}/conv_layer5", [(f"{pre}/conv_layer5/W", 64, 0, 64 + 4 * g_, 0)], 64 + 4 * g_, 64,
-                                  P[f"{pre}/conv_layer5/b"])
+                                  f"{pre}/conv_layer5/b")
                         if g_ == 32:
-                            for k in (1, 3):
-                                cin = 64 + (k - 1) * 32
-                                add_split(f"{pre}/pair{k}", [(f"{pre}/conv_layer{k}/W", 32, 0, cin, 0),
-                                                             (f"{pre}/conv_layer{k + 1}/W", 32, 32, cin + 32, 0)], cin, 64,
-                                          P[f"{pre}/conv_layer{k}/b"])
-                                add_split(f"{pre}/tail{k + 1}", [(f"{pre}/conv_layer{k + 1}/W", 32, 0, cin + 32, cin)], 32,
-                                          32, P[f"{pre}/conv_layer{k + 1}/b"])
+                            for name, slices, cin, coutp, bias in pair_images(pre):
+                                add_split(name, slices, cin, coutp, bias)
                         else:
                             for k in (1, 2, 3, 4):
                                 cin = 64 + (k - 1) * g_
                                 add_split(f"{pre}/conv_layer{k}", [(f"{pre}/conv_layer{k}/W", g_, 0, cin, 0)], cin, g_,
-                                          P[f"{pre}/conv_layer{k}/b"])
+                                          f"{pre}/conv_layer{k}/b")
             for key in ("post_upsample_conv_layer_1", "post_upsample_conv_layer_2"):
                 add(key, 64)
             add("final_conv_layer1/offset_conv", 32)
@@ -737,9 +738,7 @@ class GeneratorModel(_Link):
             return ws
         bf = torch.bfloat16
         g = self.inter_channels
-        cc = 64 + 4 * g
-        ccs = cc // 8
-        beta = self.residual_scaling
+        ccs = (64 + 4 * g) // 8
         # pairing keeps partial sums in tensor memory between a head and its tail on the same CTA; the schedule's
         # deadlock-freedom argument needs a unit's neighbours (+- one row of 16-pixel-wide units) to lie within one
         # round of CTAs, i.e. images narrower than ~2000 px (csrc/umma_trunk.cu, "schedule")
@@ -748,67 +747,33 @@ class GeneratorModel(_Link):
             ws = dict(s0=ops.empty(n, 16, H, W, 8, dtype=bf), cat=[ops.empty(n, ccs, H, W, 8, dtype=bf) for _ in range(2)],
                       a1_f32=ops.empty(n, 16, H, W, 4), f32=[ops.empty(n, 16, H, W, 4) for _ in range(3)],
                       u1=ops.empty(n, 8, 2 * H, 2 * W, 8, dtype=bf))
-        cat, f32, a1_f32 = ws["cat"], ws["f32"], ws["a1_f32"]
-        layers = []
-        flops = []
-
-        def layer(wkey, cin, cout, in_map, act=0, beta_=0.0, out=None, out_cs0=0, out_f32=None, res1=None, res2=None,
-                  up2=0, in_cs0=0, cout_main=None, res1_cs=16, stash_out=None, raw=False, mode=0):
-            trunk_pack = self.persistent_trunk or self.per_layer_ck16
-            wq, bq = pk[wkey] if raw else (pk[wkey + "@trunk"] if trunk_pack else pk[wkey])
-            ptr = lambda t: t.data_ptr() if t is not None else 0
-            layers.append((wq.data_ptr(), bq.data_ptr(), ptr(out), ptr(out_f32), ptr(res1), ptr(res2), ptr(stash_out),
-                           cin, cout, in_map, in_cs0, act, up2, out.shape[1] if out is not None else 0, out_cs0,
-                           cout if cout_main is None else cout_main, res1_cs, beta_, mode, (0,) * 6))
-            flops.append(2.0 * 9 * cin * cout * n * H * W)
-
-        layer("pre_residual_conv_layer", 128, 64, 0, act=1, out=cat[0], out_f32=a1_f32)
-        cur, cur_f32, fi = 0, a1_f32, 0
-        for i in range(self.num_residual_blocks):
-            rrdb_in = cur_f32
-            for r in (1, 2, 3):
-                pre = self._rdb_prefix(i, r)
-                if paired:
-                    # a_k = lrelu(conv_k([a0..a_{k-1}])) for k = 1..4 (srgan_train.py:339-352) in four passes:
-                    #   k odd  ("head", mode 1): N = 64 over [a0..a_{k-1}] -> a_k (32 columns, fused epilogue); the
-                    #           other 32 columns -- the partial sums of conv_{k+1} over the same inputs -- stay in
-                    #           tensor memory
-                    #   k even ("tail", mode 2): N = 32 over a_{k-1} only, accumulated onto those columns -> a_k
-                    # Same FLOPs; 252 N=32 MMAs per 128-pixel tile become 108 N=64 + 36 N=32 MMAs (each MMA
-                    # re-reads its 4 KB A operand from shared memory whatever N is), and nothing but the bf16
-                    # features a_k ever leaves the SM.
-                    for k in (1, 3):
-                        cin = 64 + (k - 1) * g
-                        if k not in self.paired_convs:     # A/B: this pair as two layers of their own
-                            for kk in (k, k + 1):
-                                ci = 64 + (kk - 1) * g
-                                layer(f"{pre}/conv_layer{kk}", ci, g, 1 + cur, act=1, out=cat[cur], out_cs0=ci // 8)
-                            continue
-                        layer(f"{pre}/pair{k}", cin, 64, 1 + cur, act=1, out=cat[cur], out_cs0=cin // 8, cout_main=32,
-                              raw=True, mode=1)
-                        layer(f"{pre}/tail{k + 1}", 32, 32, 1 + cur, in_cs0=cin // 8, act=1, out=cat[cur],
-                              out_cs0=cin // 8 + 4, raw=True, mode=2)
-                else:
-                    for k in (1, 2, 3, 4):
-                        cin = 64 + (k - 1) * g
-                        layer(f"{pre}/conv_layer{k}", cin, g, 1 + cur, act=1, out=cat[cur], out_cs0=cin // 8)
-                # fp32 residual buffer that is neither the RDB input nor the RRDB input
-                while f32[fi] is cur_f32 or f32[fi] is rrdb_in:
-                    fi = (fi + 1) % 3
-                nxt_f32 = f32[fi]
-                layer(f"{pre}/conv_layer5", cc, 64, 1 + cur, beta_=beta, out=cat[1 - cur], out_f32=nxt_f32, res1=cur_f32,
-                      res2=rrdb_in if r == 3 else None)
-                cur, cur_f32 = 1 - cur, nxt_f32
-        layer("post_residual_conv_layer", 64, 64, 1 + cur, beta_=1.0, out=ws["u1"], res1=a1_f32, up2=1)
+        plan = layout.trunk_plan(self.num_residual_blocks, g, self.residual_scaling, paired, self.paired_convs)
+        # the pair / tail images (modes 1, 2) exist in one form; the persistent kernel (and the per-layer kernel with
+        # per_layer_ck16) streams the other filters in 16-channel chunks
+        suffix = "@trunk" if self.persistent_trunk or self.per_layer_ck16 else ""
+        layers = self._bind_trunk_plan(plan, lambda p: pk[p["image"] + ("" if p["mode"] else suffix)][0], ws, 1)
         table = np.array(layers, dtype=TRUNK_LAYER_DTYPE)
         ws["layers"] = layers
-        ws["flops"] = float(sum(flops))  # executed MMA FLOPs (= algorithmic: pairing moves work, it adds none)
+        # executed MMA FLOPs (= algorithmic: pairing moves work, it adds none)
+        ws["flops"] = float(sum(2.0 * 9 * p["cin"] * p["cout"] * n * H * W for p in plan))
         ws["table"] = torch.from_numpy(table.view(np.uint8).copy()).cuda()
         tiles = ((H + 31) // 32) * ((W + 15) // 16)   # 32-row x 16-column units (kTH x kTW in umma_trunk.cu)
         ws["flags"] = ops.empty(len(layers) * n * tiles, dtype=torch.int32)
         ws["version"] = (self._pack_gen, self.persistent_trunk, self.paired_trunk, self.per_layer_ck16, self.paired_convs)
         self._ws[key] = ws
         return ws
+
+    def _bind_trunk_plan(self, plan, image, ws, slabs_per_cs):
+        """TrunkLayer rows (TRUNK_LAYER_DTYPE) of layout.trunk_plan records: ``image(p)`` is the packed filter image of
+        pass p, its buffer names are the workspace's tensors. ``out_cs_total`` counts logical slabs, out.shape[1] //
+        ``slabs_per_cs`` (2 for the split path, whose buffers hold a hi and a lo slab per logical slab)."""
+        bufs = dict(cat0=ws["cat"][0], cat1=ws["cat"][1], a1=ws["a1_f32"],
+                    **{f"f32_{i}": t for i, t in enumerate(ws["f32"])}, **{k: ws[k] for k in ("u1", "u2", "c2f") if k in ws})
+        ptr = lambda name: bufs[name].data_ptr() if name is not None else 0
+        return [(image(p).data_ptr(), self.p[p["bias"]].data_ptr(), ptr(p["out"]), ptr(p["out_f32"]), ptr(p["res1"]),
+                 ptr(p["res2"]), 0, p["cin"], p["cout"], p["in_map"], p["in_cs0"], p["act"], p["up2"],
+                 bufs[p["out"]].shape[1] // slabs_per_cs if p["out"] is not None else 0, p["out_cs0"], p["cout_main"], 16,
+                 p["beta"], p["mode"], (0,) * 6) for p in plan]
 
     def _run_trunk(self, ws, n, H, W):
         if self.persistent_trunk:
@@ -901,54 +866,22 @@ class GeneratorModel(_Link):
             return ws
         bf = torch.bfloat16
         g = self.inter_channels
-        cc = 64 + 4 * g
-        ccs = cc // 8
-        beta = self.residual_scaling
+        ccs = (64 + 4 * g) // 8
         if ws is None:
             ws = dict(s0=ops.empty(n, 32, H, W, 8, dtype=bf), cat=[ops.empty(n, 2 * ccs, H, W, 8, dtype=bf) for _ in range(2)],
                       a1_f32=ops.empty(n, 16, H, W, 4), f32=[ops.empty(n, 16, H, W, 4) for _ in range(3)],
                       u1=ops.empty(n, 16, 2 * H, 2 * W, 8, dtype=bf), u2=ops.empty(n, 16, 4 * H, 4 * W, 8, dtype=bf),
                       c2f=ops.empty(n, 16, 4 * H, 4 * W, 4))
-        cat, f32, a1_f32 = ws["cat"], ws["f32"], ws["a1_f32"]
         paired = g == 32 and (W + 15) // 16 + 2 <= 128
-
-        def rec(wkey, cin, cout, in_map, act=0, beta_=0.0, out=None, out_cs0=0, out_f32=None, res1=None, res2=None,
-                up2=0, in_cs0=0, cout_main=None, mode=0):
-            wq, bq = pk[wkey + "@split"]
-            ptr = lambda t: t.data_ptr() if t is not None else 0
-            # out_cs_total is LOGICAL (the buffers hold a hi and a lo slab per logical slab)
-            return (wq.data_ptr(), bq.data_ptr(), ptr(out), ptr(out_f32), ptr(res1), ptr(res2), 0, cin, cout, in_map,
-                    in_cs0, act, up2, out.shape[1] // 2 if out is not None else 0, out_cs0,
-                    cout if cout_main is None else cout_main, 16, beta_, mode, (0,) * 6)
-
-        layers = [rec("pre_residual_conv_layer", 128, 64, 0, act=1, out=cat[0], out_f32=a1_f32)]
-        cur, cur_f32, fi = 0, a1_f32, 0
-        for i in range(self.num_residual_blocks):
-            rrdb_in = cur_f32
-            for r in (1, 2, 3):
-                pre = self._rdb_prefix(i, r)
-                if paired:
-                    for k in (1, 3):
-                        cin = 64 + (k - 1) * g
-                        layers.append(rec(f"{pre}/pair{k}", cin, 64, 1 + cur, act=1, out=cat[cur], out_cs0=cin // 8,
-                                          cout_main=32, mode=1))
-                        layers.append(rec(f"{pre}/tail{k + 1}", 32, 32, 1 + cur, in_cs0=cin // 8, act=1, out=cat[cur],
-                                          out_cs0=cin // 8 + 4, mode=2))
-                else:
-                    if g == 32:   # only the paired images are packed for the split path
-                        raise ValueError("precision='bf16x3': tiles wider than ~2000 px are not supported")
-                    for k in (1, 2, 3, 4):
-                        cin = 64 + (k - 1) * g
-                        layers.append(rec(f"{pre}/conv_layer{k}", cin, g, 1 + cur, act=1, out=cat[cur], out_cs0=cin // 8))
-                while f32[fi] is cur_f32 or f32[fi] is rrdb_in:
-                    fi = (fi + 1) % 3
-                nxt_f32 = f32[fi]
-                layers.append(rec(f"{pre}/conv_layer5", cc, 64, 1 + cur, beta_=beta, out=cat[1 - cur], out_f32=nxt_f32,
-                                  res1=cur_f32, res2=rrdb_in if r == 3 else None))
-                cur, cur_f32 = 1 - cur, nxt_f32
-        layers.append(rec("post_residual_conv_layer", 64, 64, 1 + cur, beta_=1.0, out=ws["u1"], res1=a1_f32, up2=1))
-        up1 = [rec("post_upsample_conv_layer_1", 64, 64, 0, act=1, out=ws["u2"], up2=1)]
-        up2 = [rec("post_upsample_conv_layer_2", 64, 64, 0, act=1, out_f32=ws["c2f"])]
+        if g == 32 and not paired:   # only the paired images are packed for the split path
+            raise ValueError("precision='bf16x3': tiles wider than ~2000 px are not supported")
+        image = lambda p: pk[p["image"] + "@split"][0]
+        layers = self._bind_trunk_plan(layout.trunk_plan(self.num_residual_blocks, g, self.residual_scaling, paired),
+                                       image, ws, 2)
+        up1 = self._bind_trunk_plan([layout.trunk_pass("post_upsample_conv_layer_1", 64, 64, 0, act=1, out="u2", up2=1)],
+                                    image, ws, 2)
+        up2 = self._bind_trunk_plan([layout.trunk_pass("post_upsample_conv_layer_2", 64, 64, 0, act=1, out_f32="c2f")],
+                                    image, ws, 2)
         dev = lambda rows: torch.from_numpy(np.array(rows, dtype=TRUNK_LAYER_DTYPE).view(np.uint8).copy()).cuda()
         units = lambda h_, w_: n * ((h_ + 31) // 32) * ((w_ + 15) // 16)
         ws.update(tables=[dev(layers), dev(up1), dev(up2)], counts=[len(layers), 1, 1],

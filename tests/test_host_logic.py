@@ -46,3 +46,39 @@ def test_s2d_tap_mask_matches_the_embedding():
         assert s2d_tap_mask(ph * C + 16, 32, C) == want
     assert s2d_tap_mask(0, 128, C) == s2d_tap_mask(0, 64, C) | s2d_tap_mask(64, 64, C)
     assert s2d_tap_mask(0, 4 * C, C) == 0x1FF
+
+
+def test_trunk_plan_pass_sequence():
+    """layout.trunk_plan, the trunk pass plan both table builders bind: 2 + 15 nb passes; pair heads / tails (modes 1, 2)
+    only when paired at inter_channels 32; no conv5 writes an fp32 buffer it reads; the RRDB skip (res2) exactly on the
+    third dense block of each RRDB; and the nb = 1 paired plan, written out."""
+    from deepbedmap_b200.layout import trunk_plan
+    for nb in (1, 2, 5):
+        for inter in (32, 64):
+            for paired in (False, True):
+                for convs in ((1, 3), (3,), ()):
+                    plan = trunk_plan(nb, inter, 0.1, paired and inter == 32, convs)
+                    assert len(plan) == 2 + 15 * nb
+                    modes = {p["mode"] for p in plan}
+                    assert modes == ({0, 1, 2} if paired and inter == 32 and convs else {0})
+                    for p in plan:
+                        assert p["out_f32"] is None or p["out_f32"] not in (p["res1"], p["res2"])
+                        assert (p["res2"] is not None) == p["image"].endswith("residual_dense_block3/conv_layer5")
+    fields = ("image", "bias", "cin", "cout", "in_map", "in_cs0", "act", "up2", "out", "out_cs0", "cout_main", "beta",
+              "mode", "out_f32", "res1", "res2")
+    want = [("pre_residual_conv_layer", "pre_residual_conv_layer/b", 128, 64, 0, 0, 1, 0, "cat0", 0, 64, 0.0, 0, "a1",
+             None, None)]
+    cat, ring = ["cat0", "cat1", "cat0", "cat1"], [None, "f32_0", "f32_1", "f32_2"]
+    res1 = ["a1", "f32_0", "f32_1"]
+    for r in (1, 2, 3):
+        pre = f"residual_network/0/residual_dense_block{r}"
+        c, m = cat[r - 1], 1 + (r - 1) % 2
+        want += [(f"{pre}/pair1", f"{pre}/conv_layer1/b", 64, 64, m, 0, 1, 0, c, 8, 32, 0.0, 1, None, None, None),
+                 (f"{pre}/tail2", f"{pre}/conv_layer2/b", 32, 32, m, 8, 1, 0, c, 12, 32, 0.0, 2, None, None, None),
+                 (f"{pre}/pair3", f"{pre}/conv_layer3/b", 128, 64, m, 0, 1, 0, c, 16, 32, 0.0, 1, None, None, None),
+                 (f"{pre}/tail4", f"{pre}/conv_layer4/b", 32, 32, m, 16, 1, 0, c, 20, 32, 0.0, 2, None, None, None),
+                 (f"{pre}/conv_layer5", f"{pre}/conv_layer5/b", 192, 64, m, 0, 0, 0, cat[r], 0, 64, 0.25, 0, ring[r],
+                  res1[r - 1], "a1" if r == 3 else None)]
+    want.append(("post_residual_conv_layer", "post_residual_conv_layer/b", 64, 64, 2, 0, 0, 1, "u1", 0, 64, 1.0, 0, None,
+                 "a1", None))
+    assert [tuple(p[f] for f in fields) for p in trunk_plan(1, 32, 0.25, True)] == want
